@@ -130,6 +130,24 @@ def test_zero_padding_large_rotation():
     assert np.abs(warped - co.warp_affine(mov.numpy(), th.cpu().numpy())).max() < 1e-5
 
 
+def test_forward_warp_tma_kernel_equals_gather_kernel():
+    """3-D forward warp: the TMA-staged kernel (small angles) against the one-thread-per-voxel gather kernel
+    (large_rotation=True), over 3 pairs x 2 channels of a shape with partial tiles along every axis.  The 45-degree theta
+    misses the staged box, so those tiles take the TMA kernel's global-gather fallback."""
+    TF = _tf()
+    from torchregister_b200.synth import make_pair
+    m, _ = make_pair((37, 50, 68), "flow")
+    m = m.to(DEV)
+    batch = torch.cat([torch.cat([m, 0.5 * m + 0.1], 1), torch.cat([0.3 * m, m * m], 1), torch.cat([m, -m], 1)], 0).contiguous()
+    small = torch.tensor([[1.01, .02, -.01, .01], [-.02, .99, .01, 0.], [.01, -.01, 1., .02]], device=DEV)
+    big = torch.tensor([[0.7, -0.7, 0.1, .05], [0.7, 0.7, -0.1, 0.], [0.0, 0.14, 0.99, .02]], device=DEV)
+    ths = torch.stack([small, big, small * 0.98])
+    tma = TF.warp_affine(ths, batch)
+    gather = TF.warp_affine(ths, batch, large_rotation=True)
+    # the two kernels form the source coordinate with different fp32 operation chains
+    assert (tma - gather).abs().max().item() < 1e-5
+
+
 def test_batch_equals_singles_and_is_deterministic():
     TF = _tf()
     from torchregister_b200.synth import make_pair

@@ -728,14 +728,12 @@ affine3d_persist_kernel(const PersistParams pp, const __grid_constant__ CUtensor
                         const float2 iz = __ffma2_rn(f2(sz[2]), zf, f2(pxy[2]));
                         // immediates: the target tile advances TX*TY*4 bytes per z
                         const float2 t = make_float2(lds_f<(2 * j) * TX * TY * 4>(tg), lds_f<(2 * j + 1) * TX * TY * 4>(tg));
+                        const float2 wv = pair_step2<kBX, kBY, true, MSE_ONLY>(box_addr, Mrel, ix, iy, iz, t, zf, A);
                         if constexpr (STORE) {
-                            const float2 wv = pair_step2w<kBX, kBY, true, MSE_ONLY>(box_addr, Mrel, ix, iy, iz, t, zf, A);
                             const size_t HWs = (size_t)H * W;
                             float *wz = wcol0 + (size_t)(int)zf0 * HWs;
                             __stcs(wz + (size_t)(2 * j) * HWs, wv.x);
                             __stcs(wz + (size_t)(2 * j + 1) * HWs, wv.y);
-                        } else {
-                            pair_step2<kBX, kBY, true, MSE_ONLY>(box_addr, Mrel, ix, iy, iz, t, zf, A);
                         }
                         zf = __fadd2_rn(zf, f2(2.f));
                     });
@@ -752,16 +750,13 @@ affine3d_persist_kernel(const PersistParams pp, const __grid_constant__ CUtensor
                         const float2 iz = __ffma2_rn(f2(sz[2]), zf, f2(pxy[2]));
                         const float2 t = make_float2(lds_f_dyn(tg + zz * (TX * TY * 4)),
                                                      lds_f_dyn(tg + (second ? zz + 1 : zz) * (TX * TY * 4)));
+                        const float2 wv = second ? pair_step2<kBX, kBY, true, MSE_ONLY>(box_addr, Mrel, ix, iy, iz, t, zf, A)
+                                                 : pair_step2<kBX, kBY, false, MSE_ONLY>(box_addr, Mrel, ix, iy, iz, t, zf, A);
                         if constexpr (STORE) {
-                            const float2 wv = second ? pair_step2w<kBX, kBY, true, MSE_ONLY>(box_addr, Mrel, ix, iy, iz, t, zf, A)
-                                                     : pair_step2w<kBX, kBY, false, MSE_ONLY>(box_addr, Mrel, ix, iy, iz, t, zf, A);
                             const size_t HWs = (size_t)H * W;
                             float *wz = wcol0 + (size_t)(int)zf0 * HWs;
                             __stcs(wz + (size_t)zz * HWs, wv.x);
                             if (second) __stcs(wz + (size_t)(zz + 1) * HWs, wv.y);
-                        } else {
-                            if (second) pair_step2<kBX, kBY, true, MSE_ONLY>(box_addr, Mrel, ix, iy, iz, t, zf, A);
-                            else pair_step2<kBX, kBY, false, MSE_ONLY>(box_addr, Mrel, ix, iy, iz, t, zf, A);
                         }
                     }
                 }

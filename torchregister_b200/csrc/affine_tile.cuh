@@ -1,7 +1,9 @@
 // affine_tile.cuh — device pieces shared by the TMA-staged 3-D rigid/affine kernels (sm_100a):
 // affine_tma.cu (one launch per epoch; also the unfused moments pass) and affine_persist.cu (persistent,
-// warp-specialised multi-epoch kernel).  PTX wrappers, the per-voxel-pair arithmetic (pair_step), the global-gather
-// fallback, the work decomposition (TileIter), the footprint bound and the tensor-map encoder.
+// warp-specialised multi-epoch kernel), and by the forward warp (warp_tma.cu).  PTX wrappers, the staged-box sampling
+// (box_cells, pair_sample, voxel_staged) and the moment accumulation over it (pair_step, pair_step2), the clamped global
+// gather of the fallback paths (gather_clamped3), the work decomposition (TileIter), the footprint bound and the
+// tensor-map encoder.  The scalar blend itself is common.cuh's blend_cell3.
 #pragma once
 #include "common.cuh"
 #include "affine_shared.cuh"
@@ -143,25 +145,42 @@ struct Acc {
     float2 Q[3][3];     // sum k*G_r*z
 };
 
-// one pair of voxels (same x,y; z and z+1).  box_m: smem byte address of the staged box.
-// SECOND=false masks voxel b.
-template <int BX, int BY, bool SECOND, bool MSE_ONLY>
-__device__ __forceinline__ float2 pair_step(uint32_t box_m, float Mrel, float2 ix, float2 iy, float2 iz,
-                                            float2 t, float2 zf, Acc &A)
+// Staged-box cells of two voxels (same x,y; z and z+1): fractions and box indices.
+// floor() = round-down add of 1.5*2^23 (FADD.RM) and subtracting it again; FRND on the XU pipe was
+// tried instead (it frees 6 packed fp32 ops per pair) but its latency lengthened the dependent
+// chain and the step got 11% slower (profiles/r01_notes.md)
+struct BoxCells {
+    float2 tx, ty, tz;      // fractions (voxel a, voxel b)
+    float2 tb;              // box indices of the two cells' (x0,y0,z0) corners, see cell_addr
+};
+template <int BX, int BY>
+__device__ __forceinline__ BoxCells box_cells(float Mrel, float2 ix, float2 iy, float2 iz)
 {
-    // floor() = round-down add of 1.5*2^23 (FADD.RM) and subtracting it again; FRND on the XU pipe was
-    // tried instead (it frees 6 packed fp32 ops per pair) but its latency lengthened the dependent
-    // chain and the step got 11% slower (profiles/r01_notes.md)
+    BoxCells b;
     const float2 M = f2(kMagic), nM = f2(-kMagic);
     const float2 flx = __fadd2_rd(ix, M), fly = __fadd2_rd(iy, M), flz = __fadd2_rd(iz, M);
     const float2 fx = __fadd2_rn(flx, nM), fy = __fadd2_rn(fly, nM), fz = __fadd2_rn(flz, nM);
-    const float2 tx = sub2(ix, fx), ty = sub2(iy, fy), tz = sub2(iz, fz);
-    // box-relative linear index, formed in fp32 and scaled by 2^-22 onto [2, 4): exact, and the bit
-    // pattern is 0x40000000 + index, so (bits << 2) IS the byte offset (the 0x4 wraps away)
-    const float2 tb = __ffma2_rn(f2(kIdxScale * (float)(BX * BY)), fz,
-                                 __ffma2_rn(f2(kIdxScale * (float)BX), fy, __ffma2_rn(f2(kIdxScale), fx, f2(Mrel))));
-    const uint32_t qa = box_m + ((uint32_t)__float_as_int(tb.x) << 2);
-    const uint32_t qb = box_m + ((uint32_t)__float_as_int(tb.y) << 2);
+    b.tx = sub2(ix, fx); b.ty = sub2(iy, fy); b.tz = sub2(iz, fz);
+    b.tb = __ffma2_rn(f2(kIdxScale * (float)(BX * BY)), fz,
+                      __ffma2_rn(f2(kIdxScale * (float)BX), fy, __ffma2_rn(f2(kIdxScale), fx, f2(Mrel))));
+    return b;
+}
+// smem byte address of a cell's corner; box_m: smem byte address of the staged box.  The box-relative linear index
+// is formed in fp32 and scaled by 2^-22 onto [2, 4): exact, and the bit pattern is 0x40000000 + index, so (bits << 2)
+// IS the byte offset (the 0x4 wraps away)
+__device__ __forceinline__ uint32_t cell_addr(uint32_t box_m, float tb) { return box_m + ((uint32_t)__float_as_int(tb) << 2); }
+
+// trilinear sample of both voxels from the staged box, packed (voxel a, voxel b) in every value;
+// g: d val / d (x, y, z) in voxel units (WANT_GRAD only)
+struct PairSample {
+    float2 val, g[3];
+};
+template <int BX, int BY, bool WANT_GRAD>
+__device__ __forceinline__ PairSample pair_sample(uint32_t box_m, const BoxCells &b)
+{
+    PairSample s;
+    const uint32_t qa = cell_addr(box_m, b.tb.x), qb = cell_addr(box_m, b.tb.y);
+    const float2 tx = b.tx, ty = b.ty, tz = b.tz;
     constexpr int SY = BX * 4, SZ = BX * BY * 4;
     const float2 c000 = make_float2(lds_f<0>(qa), lds_f<0>(qb)), c001 = make_float2(lds_f<4>(qa), lds_f<4>(qb));
     const float2 c010 = make_float2(lds_f<SY>(qa), lds_f<SY>(qb)), c011 = make_float2(lds_f<SY + 4>(qa), lds_f<SY + 4>(qb));
@@ -173,12 +192,25 @@ __device__ __forceinline__ float2 pair_step(uint32_t box_m, float Mrel, float2 i
     const float2 v10 = __ffma2_rn(tx, d10, c100), v11 = __ffma2_rn(tx, d11, c110);
     const float2 e0 = sub2(v01, v00), e1 = sub2(v11, v10);
     const float2 w0 = __ffma2_rn(ty, e0, v00), w1 = __ffma2_rn(ty, e1, v10);
-    float2 G[3];
-    G[2] = sub2(w1, w0);
-    float2 val = __ffma2_rn(tz, G[2], w0);
-    G[1] = __ffma2_rn(tz, sub2(e1, e0), e0);
-    const float2 dx0 = __ffma2_rn(ty, sub2(d01, d00), d00), dx1 = __ffma2_rn(ty, sub2(d11, d10), d10);
-    G[0] = __ffma2_rn(tz, sub2(dx1, dx0), dx0);
+    const float2 gz = sub2(w1, w0);
+    s.val = __ffma2_rn(tz, gz, w0);
+    if (WANT_GRAD) {
+        s.g[2] = gz;
+        s.g[1] = __ffma2_rn(tz, sub2(e1, e0), e0);
+        const float2 dx0 = __ffma2_rn(ty, sub2(d01, d00), d00), dx1 = __ffma2_rn(ty, sub2(d11, d10), d10);
+        s.g[0] = __ffma2_rn(tz, sub2(dx1, dx0), dx0);
+    }
+    return s;
+}
+
+// one pair of voxels (same x,y; z and z+1) into the round-1 accumulators.  SECOND=false masks voxel b.
+template <int BX, int BY, bool SECOND, bool MSE_ONLY>
+__device__ __forceinline__ float2 pair_step(uint32_t box_m, float Mrel, float2 ix, float2 iy, float2 iz,
+                                            float2 t, float2 zf, Acc &A)
+{
+    const PairSample s = pair_sample<BX, BY, true>(box_m, box_cells<BX, BY>(Mrel, ix, iy, iz));
+    float2 G[3] = {s.g[0], s.g[1], s.g[2]};
+    float2 val = s.val;
     if (!SECOND) {                       // odd tail: the duplicate voxel contributes nothing
         const float2 m = make_float2(1.f, 0.f);
         val = __fmul2_rn(val, m); t = __fmul2_rn(t, m);
@@ -267,53 +299,9 @@ __device__ __forceinline__ void moments_accumulate(float t, float z, float val, 
     }
 }
 
-// one voxel whose cell is staged in shared memory at byte address q (its corner (x0,y0,z0))
+// one voxel whose cell is staged in shared memory at byte address q (its corner (x0,y0,z0)); returns the warped sample
 template <int BX, int BY, bool MSE_ONLY>
-__device__ __forceinline__ void voxel_staged(uint32_t q, float tx, float ty, float tz, float t, float z, Acc2 &A)
-{
-    constexpr int SY = BX * 4, SZ = BX * BY * 4;
-    const float2 P0 = make_float2(lds_f<0>(q), lds_f<SZ>(q)), P1 = make_float2(lds_f<4>(q), lds_f<SZ + 4>(q));
-    const float2 R0 = make_float2(lds_f<SY>(q), lds_f<SZ + SY>(q)), R1 = make_float2(lds_f<SY + 4>(q), lds_f<SZ + SY + 4>(q));
-    const float2 dP = sub2(P1, P0), dR = sub2(R1, R0);                   // (d00, d10), (d01, d11)
-    const float2 vA = __ffma2_rn(f2(tx), dP, P0), vB = __ffma2_rn(f2(tx), dR, R0);   // (v00, v10), (v01, v11)
-    const float2 e = sub2(vB, vA);                                        // (e0, e1)
-    const float2 w = __ffma2_rn(f2(ty), e, vA);                           // (w0, w1)
-    const float2 dx = __ffma2_rn(f2(ty), sub2(dR, dP), dP);               // (dx0, dx1)
-    const float G2 = w.y - w.x;
-    const float val = fmaf(tz, G2, w.x);
-    const float G1 = fmaf(tz, e.y - e.x, e.x);
-    const float G0 = fmaf(tz, dx.y - dx.x, dx.x);
-    moments_accumulate<MSE_ONLY>(t, z, val, G0, G1, G2, A);
-}
-
-// two voxels (same x,y; z and z+1): coordinates, floor, fraction and index stay packed over the two voxels (their
-// operands are per-thread constants, i.e. broadcasts); SECOND = false skips voxel b.
-template <int BX, int BY, bool SECOND, bool MSE_ONLY>
-__device__ __forceinline__ void pair_step2(uint32_t box_m, float Mrel, float2 ix, float2 iy, float2 iz, float2 t, float2 zf, Acc2 &A)
-{
-#ifdef TRB_XU_FLOOR
-    // floor on the (otherwise idle) XU pipe: FRND.FLOOR, 16 lanes/clk/SM, instead of two packed adds on the fp32 pipe
-    const float2 fx = make_float2(floorf(ix.x), floorf(ix.y)), fy = make_float2(floorf(iy.x), floorf(iy.y)),
-                 fz = make_float2(floorf(iz.x), floorf(iz.y));
-#else
-    const float2 M = f2(kMagic), nM = f2(-kMagic);
-    const float2 flx = __fadd2_rd(ix, M), fly = __fadd2_rd(iy, M), flz = __fadd2_rd(iz, M);
-    const float2 fx = __fadd2_rn(flx, nM), fy = __fadd2_rn(fly, nM), fz = __fadd2_rn(flz, nM);
-#endif
-    const float2 tx = sub2(ix, fx), ty = sub2(iy, fy), tz = sub2(iz, fz);
-    const float2 tb = __ffma2_rn(f2(kIdxScale * (float)(BX * BY)), fz,
-                                 __ffma2_rn(f2(kIdxScale * (float)BX), fy, __ffma2_rn(f2(kIdxScale), fx, f2(Mrel))));
-    const uint32_t qa = box_m + ((uint32_t)__float_as_int(tb.x) << 2);
-    voxel_staged<BX, BY, MSE_ONLY>(qa, tx.x, ty.x, tz.x, t.x, zf.x, A);
-    if (SECOND) {
-        const uint32_t qb = box_m + ((uint32_t)__float_as_int(tb.y) << 2);
-        voxel_staged<BX, BY, MSE_ONLY>(qb, tx.y, ty.y, tz.y, t.y, zf.y, A);
-    }
-}
-
-// the same two functions returning the warped sample(s) (unfused pass that also stores the warped volume)
-template <int BX, int BY, bool MSE_ONLY>
-__device__ __forceinline__ float voxel_staged_w(uint32_t q, float tx, float ty, float tz, float t, float z, Acc2 &A)
+__device__ __forceinline__ float voxel_staged(uint32_t q, float tx, float ty, float tz, float t, float z, Acc2 &A)
 {
     constexpr int SY = BX * 4, SZ = BX * BY * 4;
     const float2 P0 = make_float2(lds_f<0>(q), lds_f<SZ>(q)), P1 = make_float2(lds_f<4>(q), lds_f<SZ + 4>(q));
@@ -332,31 +320,30 @@ __device__ __forceinline__ float voxel_staged_w(uint32_t q, float tx, float ty, 
 }
 
 // two voxels (same x,y; z and z+1): coordinates, floor, fraction and index stay packed over the two voxels (their
-// operands are per-thread constants, i.e. broadcasts); SECOND = false skips voxel b.
+// operands are per-thread constants, i.e. broadcasts); SECOND = false skips voxel b.  Returns the two warped samples.
 template <int BX, int BY, bool SECOND, bool MSE_ONLY>
-__device__ __forceinline__ float2 pair_step2w(uint32_t box_m, float Mrel, float2 ix, float2 iy, float2 iz, float2 t, float2 zf, Acc2 &A)
+__device__ __forceinline__ float2 pair_step2(uint32_t box_m, float Mrel, float2 ix, float2 iy, float2 iz, float2 t, float2 zf, Acc2 &A)
 {
-#ifdef TRB_XU_FLOOR
-    // floor on the (otherwise idle) XU pipe: FRND.FLOOR, 16 lanes/clk/SM, instead of two packed adds on the fp32 pipe
-    const float2 fx = make_float2(floorf(ix.x), floorf(ix.y)), fy = make_float2(floorf(iy.x), floorf(iy.y)),
-                 fz = make_float2(floorf(iz.x), floorf(iz.y));
-#else
-    const float2 M = f2(kMagic), nM = f2(-kMagic);
-    const float2 flx = __fadd2_rd(ix, M), fly = __fadd2_rd(iy, M), flz = __fadd2_rd(iz, M);
-    const float2 fx = __fadd2_rn(flx, nM), fy = __fadd2_rn(fly, nM), fz = __fadd2_rn(flz, nM);
-#endif
-    const float2 tx = sub2(ix, fx), ty = sub2(iy, fy), tz = sub2(iz, fz);
-    const float2 tb = __ffma2_rn(f2(kIdxScale * (float)(BX * BY)), fz,
-                                 __ffma2_rn(f2(kIdxScale * (float)BX), fy, __ffma2_rn(f2(kIdxScale), fx, f2(Mrel))));
-    const uint32_t qa = box_m + ((uint32_t)__float_as_int(tb.x) << 2);
-    float2 w;                            // the two warped samples (z, z + 1)
-    w.x = voxel_staged_w<BX, BY, MSE_ONLY>(qa, tx.x, ty.x, tz.x, t.x, zf.x, A);
+    const BoxCells c = box_cells<BX, BY>(Mrel, ix, iy, iz);
+    float2 w;
+    w.x = voxel_staged<BX, BY, MSE_ONLY>(cell_addr(box_m, c.tb.x), c.tx.x, c.ty.x, c.tz.x, t.x, zf.x, A);
     w.y = 0.f;
-    if (SECOND) {
-        const uint32_t qb = box_m + ((uint32_t)__float_as_int(tb.y) << 2);
-        w.y = voxel_staged_w<BX, BY, MSE_ONLY>(qb, tx.y, ty.y, tz.y, t.y, zf.y, A);
-    }
+    if (SECOND) w.y = voxel_staged<BX, BY, MSE_ONLY>(cell_addr(box_m, c.tb.y), c.tx.y, c.ty.y, c.tz.y, t.y, zf.y, A);
     return w;
+}
+
+// Global gather for the voxels whose cell is not staged: the position is clamped to [-4, S + 4] (keeps the
+// magic-number floor in range; a clamped cell lies wholly in the zero padding), then 8 predicated loads.
+__device__ __forceinline__ Cell3 gather_clamped3(const float *__restrict__ mov, int D, int H, int W, float ix, float iy, float iz)
+{
+    Cell3 k;
+    ix = fminf(fmaxf(ix, -4.f), (float)W + 4.f);
+    iy = fminf(fmaxf(iy, -4.f), (float)H + 4.f);
+    iz = fminf(fmaxf(iz, -4.f), (float)D + 4.f);
+    k.fx = __fadd_rd(ix, kMagic) - kMagic; k.fy = __fadd_rd(iy, kMagic) - kMagic; k.fz = __fadd_rd(iz, kMagic) - kMagic;
+    k.tx = ix - k.fx; k.ty = iy - k.fy; k.tz = iz - k.fz;
+    load_cell3(mov, D, H, W, (int)k.fx, (int)k.fy, (int)k.fz, k.c);
+    return k;
 }
 
 // fallback for tiles whose source footprint does not fit the TMA box: one voxel, global gathers (Acc2 form)
@@ -364,31 +351,9 @@ template <bool MSE_ONLY>
 __device__ __forceinline__ float voxel_direct2(const float *__restrict__ mov, int D, int H, int W, float ix, float iy, float iz,
                                                float t, float zf, Acc2 &A)
 {
-    ix = fminf(fmaxf(ix, -4.f), (float)W + 4.f);        // keeps the magic-number floor in range
-    iy = fminf(fmaxf(iy, -4.f), (float)H + 4.f);
-    iz = fminf(fmaxf(iz, -4.f), (float)D + 4.f);
-    const float fx = __fadd_rd(ix, kMagic) - kMagic, fy = __fadd_rd(iy, kMagic) - kMagic, fz = __fadd_rd(iz, kMagic) - kMagic;
-    const float tx = ix - fx, ty = iy - fy, tz = iz - fz;
-    const int x0 = (int)fx, y0 = (int)fy, z0 = (int)fz;
-    const bool vx0 = (unsigned)x0 < (unsigned)W, vx1 = (unsigned)(x0 + 1) < (unsigned)W;
-    const bool vy0 = (unsigned)y0 < (unsigned)H, vy1 = (unsigned)(y0 + 1) < (unsigned)H;
-    const bool vz0 = (unsigned)z0 < (unsigned)D, vz1 = (unsigned)(z0 + 1) < (unsigned)D;
-    const long long HW = (long long)H * W, o = ((long long)z0 * H + y0) * W + x0;
-    const float c000 = (vz0 & vy0 & vx0) ? __ldg(mov + o) : 0.f, c001 = (vz0 & vy0 & vx1) ? __ldg(mov + o + 1) : 0.f;
-    const float c010 = (vz0 & vy1 & vx0) ? __ldg(mov + o + W) : 0.f, c011 = (vz0 & vy1 & vx1) ? __ldg(mov + o + W + 1) : 0.f;
-    const float c100 = (vz1 & vy0 & vx0) ? __ldg(mov + o + HW) : 0.f, c101 = (vz1 & vy0 & vx1) ? __ldg(mov + o + HW + 1) : 0.f;
-    const float c110 = (vz1 & vy1 & vx0) ? __ldg(mov + o + HW + W) : 0.f, c111 = (vz1 & vy1 & vx1) ? __ldg(mov + o + HW + W + 1) : 0.f;
-    const float d00 = c001 - c000, d01 = c011 - c010, d10 = c101 - c100, d11 = c111 - c110;
-    const float v00 = fmaf(tx, d00, c000), v01 = fmaf(tx, d01, c010), v10 = fmaf(tx, d10, c100), v11 = fmaf(tx, d11, c110);
-    const float e0 = v01 - v00, e1 = v11 - v10;
-    const float w0 = fmaf(ty, e0, v00), w1 = fmaf(ty, e1, v10);
-    const float G2 = w1 - w0;
-    const float val = fmaf(tz, G2, w0);
-    const float G1 = fmaf(tz, e1 - e0, e0);
-    const float dx0 = fmaf(ty, d01 - d00, d00), dx1 = fmaf(ty, d11 - d10, d10);
-    const float G0 = fmaf(tz, dx1 - dx0, dx0);
-    moments_accumulate<MSE_ONLY>(t, zf, val, G0, G1, G2, A);
-    return val;
+    const Sample<3> s = blend_cell3<true>(gather_clamped3(mov, D, H, W, ix, iy, iz));
+    moments_accumulate<MSE_ONLY>(t, zf, s.val, s.g[0], s.g[1], s.g[2], A);
+    return s.val;
 }
 
 // the same voxel from the PAIR volume (large-rotation variant): P[z][y][xr] = (v[xr-2], v[xr-1]) with W + 3 records per row and
@@ -411,17 +376,12 @@ __device__ __forceinline__ float voxel_direct2p(const float2 *__restrict__ P, in
     const float2 zero = make_float2(0.f, 0.f);
     const float2 r00 = (vz0 & vy0) ? __ldg(P + o) : zero, r01 = (vz0 & vy1) ? __ldg(P + o + Wp) : zero;
     const float2 r10 = (vz1 & vy0) ? __ldg(P + o + HWp) : zero, r11 = (vz1 & vy1) ? __ldg(P + o + HWp + Wp) : zero;
-    const float d00 = r00.y - r00.x, d01 = r01.y - r01.x, d10 = r10.y - r10.x, d11 = r11.y - r11.x;
-    const float v00 = fmaf(tx, d00, r00.x), v01 = fmaf(tx, d01, r01.x), v10 = fmaf(tx, d10, r10.x), v11 = fmaf(tx, d11, r11.x);
-    const float e0 = v01 - v00, e1 = v11 - v10;
-    const float w0 = fmaf(ty, e0, v00), w1 = fmaf(ty, e1, v10);
-    const float G2 = w1 - w0;
-    const float val = fmaf(tz, G2, w0);
-    const float G1 = fmaf(tz, e1 - e0, e0);
-    const float dx0 = fmaf(ty, d01 - d00, d00), dx1 = fmaf(ty, d11 - d10, d10);
-    const float G0 = fmaf(tz, dx1 - dx0, dx0);
-    moments_accumulate<MSE_ONLY>(t, zf, val, G0, G1, G2, A);
-    return val;
+    Cell3 k;
+    k.c[0] = r00.x; k.c[1] = r00.y; k.c[2] = r01.x; k.c[3] = r01.y; k.c[4] = r10.x; k.c[5] = r10.y; k.c[6] = r11.x; k.c[7] = r11.y;
+    k.tx = tx; k.ty = ty; k.tz = tz;
+    const Sample<3> s = blend_cell3<true>(k);
+    moments_accumulate<MSE_ONLY>(t, zf, s.val, s.g[0], s.g[1], s.g[2], A);
+    return s.val;
 }
 
 // and from the QUAD volume: Q[z][yr][xr] = (v[y][x], v[y][x+1], v[y+1][x], v[y+1][x+1]) at (x, y) = (xr - 2, yr - 2), H + 3 rows
@@ -441,17 +401,12 @@ __device__ __forceinline__ float voxel_direct2q(const float4 *__restrict__ Q, in
     const long long Wp = W + kPairPad, HWp = (long long)(H + kPairPad) * Wp, o = (long long)z0 * HWp + (long long)(y0 + 2) * Wp + (x0 + 2);
     const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
     const float4 q0 = vz0 ? __ldg(Q + o) : zero, q1 = vz1 ? __ldg(Q + o + HWp) : zero;      // (c00, c01, c10, c11) of plane z0 / z0 + 1
-    const float d00 = q0.y - q0.x, d01 = q0.w - q0.z, d10 = q1.y - q1.x, d11 = q1.w - q1.z;
-    const float v00 = fmaf(tx, d00, q0.x), v01 = fmaf(tx, d01, q0.z), v10 = fmaf(tx, d10, q1.x), v11 = fmaf(tx, d11, q1.z);
-    const float e0 = v01 - v00, e1 = v11 - v10;
-    const float w0 = fmaf(ty, e0, v00), w1 = fmaf(ty, e1, v10);
-    const float G2 = w1 - w0;
-    const float val = fmaf(tz, G2, w0);
-    const float G1 = fmaf(tz, e1 - e0, e0);
-    const float dx0 = fmaf(ty, d01 - d00, d00), dx1 = fmaf(ty, d11 - d10, d10);
-    const float G0 = fmaf(tz, dx1 - dx0, dx0);
-    moments_accumulate<MSE_ONLY>(t, zf, val, G0, G1, G2, A);
-    return val;
+    Cell3 k;
+    k.c[0] = q0.x; k.c[1] = q0.y; k.c[2] = q0.z; k.c[3] = q0.w; k.c[4] = q1.x; k.c[5] = q1.y; k.c[6] = q1.z; k.c[7] = q1.w;
+    k.tx = tx; k.ty = ty; k.tz = tz;
+    const Sample<3> s = blend_cell3<true>(k);
+    moments_accumulate<MSE_ONLY>(t, zf, s.val, s.g[0], s.g[1], s.g[2], A);
+    return s.val;
 }
 
 // fallback for tiles whose source footprint does not fit the TMA box: one voxel, global gathers
@@ -459,30 +414,9 @@ template <bool MSE_ONLY>
 __device__ __forceinline__ float voxel_direct(const float *__restrict__ mov, int D, int H, int W, float ix, float iy, float iz,
                                               float t, float zf, Acc &A)
 {
-    ix = fminf(fmaxf(ix, -4.f), (float)W + 4.f);        // keeps the magic-number floor in range
-    iy = fminf(fmaxf(iy, -4.f), (float)H + 4.f);
-    iz = fminf(fmaxf(iz, -4.f), (float)D + 4.f);
-    const float fx = __fadd_rd(ix, kMagic) - kMagic, fy = __fadd_rd(iy, kMagic) - kMagic, fz = __fadd_rd(iz, kMagic) - kMagic;
-    const float tx = ix - fx, ty = iy - fy, tz = iz - fz;
-    const int x0 = (int)fx, y0 = (int)fy, z0 = (int)fz;
-    const bool vx0 = (unsigned)x0 < (unsigned)W, vx1 = (unsigned)(x0 + 1) < (unsigned)W;
-    const bool vy0 = (unsigned)y0 < (unsigned)H, vy1 = (unsigned)(y0 + 1) < (unsigned)H;
-    const bool vz0 = (unsigned)z0 < (unsigned)D, vz1 = (unsigned)(z0 + 1) < (unsigned)D;
-    const long long HW = (long long)H * W, o = ((long long)z0 * H + y0) * W + x0;
-    const float c000 = (vz0 & vy0 & vx0) ? __ldg(mov + o) : 0.f, c001 = (vz0 & vy0 & vx1) ? __ldg(mov + o + 1) : 0.f;
-    const float c010 = (vz0 & vy1 & vx0) ? __ldg(mov + o + W) : 0.f, c011 = (vz0 & vy1 & vx1) ? __ldg(mov + o + W + 1) : 0.f;
-    const float c100 = (vz1 & vy0 & vx0) ? __ldg(mov + o + HW) : 0.f, c101 = (vz1 & vy0 & vx1) ? __ldg(mov + o + HW + 1) : 0.f;
-    const float c110 = (vz1 & vy1 & vx0) ? __ldg(mov + o + HW + W) : 0.f, c111 = (vz1 & vy1 & vx1) ? __ldg(mov + o + HW + W + 1) : 0.f;
-    const float d00 = c001 - c000, d01 = c011 - c010, d10 = c101 - c100, d11 = c111 - c110;
-    const float v00 = fmaf(tx, d00, c000), v01 = fmaf(tx, d01, c010), v10 = fmaf(tx, d10, c100), v11 = fmaf(tx, d11, c110);
-    const float e0 = v01 - v00, e1 = v11 - v10;
-    const float w0 = fmaf(ty, e0, v00), w1 = fmaf(ty, e1, v10);
-    float G[3];
-    G[2] = w1 - w0;
-    const float val = fmaf(tz, G[2], w0);
-    G[1] = fmaf(tz, e1 - e0, e0);
-    const float dx0 = fmaf(ty, d01 - d00, d00), dx1 = fmaf(ty, d11 - d10, d10);
-    G[0] = fmaf(tz, dx1 - dx0, dx0);
+    const Sample<3> s = blend_cell3<true>(gather_clamped3(mov, D, H, W, ix, iy, iz));
+    const float val = s.val;
+    const float *G = s.g;
     if (MSE_ONLY) {
         const float d = val - t;
         A.s[2].x = fmaf(d, d, A.s[2].x);

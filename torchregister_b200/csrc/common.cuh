@@ -99,9 +99,9 @@ __device__ __forceinline__ void floor_frac(float p, int &i0, float &t)
     floor_frac(p, i0, t, fl);
 }
 
-// cells that straddle the volume boundary (rare: kept out of line so the common path stays small)
-static __device__ __noinline__ void gather_border3(const float *__restrict__ m, int D, int H, int W, int x0, int y0, int z0,
-                                            float (&c)[8])
+// the 8 corners of the cell with origin (x0,y0,z0), zero outside the volume: predicated loads, 64-bit offsets
+__device__ __forceinline__ void load_cell3(const float *__restrict__ m, int D, int H, int W, int x0, int y0, int z0,
+                                           float (&c)[8])
 {
     const bool vx0 = (unsigned)x0 < (unsigned)W, vx1 = (unsigned)(x0 + 1) < (unsigned)W;
     const bool vy0 = (unsigned)y0 < (unsigned)H, vy1 = (unsigned)(y0 + 1) < (unsigned)H;
@@ -116,6 +116,23 @@ static __device__ __noinline__ void gather_border3(const float *__restrict__ m, 
     c[5] = (vz1 & vy0 & vx1) ? __ldg(q + HW + 1) : 0.f;
     c[6] = (vz1 & vy1 & vx0) ? __ldg(q + HW + W) : 0.f;
     c[7] = (vz1 & vy1 & vx1) ? __ldg(q + HW + W + 1) : 0.f;
+}
+// cells that straddle the volume boundary (rare: kept out of line so the common path stays small)
+static __device__ __noinline__ void gather_border3(const float *__restrict__ m, int D, int H, int W, int x0, int y0, int z0,
+                                                   float (&c)[8])
+{
+    load_cell3(m, D, H, W, x0, y0, z0, c);
+}
+// the 2-D twin: the 4 corners of the cell with origin (x0,y0)
+__device__ __forceinline__ void load_cell2(const float *__restrict__ m, int H, int W, int x0, int y0, float (&c)[4])
+{
+    const bool vx0 = (unsigned)x0 < (unsigned)W, vx1 = (unsigned)(x0 + 1) < (unsigned)W;
+    const bool vy0 = (unsigned)y0 < (unsigned)H, vy1 = (unsigned)(y0 + 1) < (unsigned)H;
+    const float *q = m + ((long long)y0 * W + x0);
+    c[0] = (vy0 & vx0) ? __ldg(q) : 0.f;
+    c[1] = (vy0 & vx1) ? __ldg(q + 1) : 0.f;
+    c[2] = (vy1 & vx0) ? __ldg(q + W) : 0.f;
+    c[3] = (vy1 & vx1) ? __ldg(q + W + 1) : 0.f;
 }
 
 template <int NDIM>
@@ -190,6 +207,26 @@ __device__ __forceinline__ Sample<3> blend_cell3(const Cell3 &k)
     return s;
 }
 
+// the 2-D twin: corners (c00, c01, c10, c11) with x fastest, and the fractions
+struct Cell2 {
+    float c[4];
+    float tx, ty;
+};
+template <bool WANT_GRAD>
+__device__ __forceinline__ Sample<2> blend_cell2(const Cell2 &k)
+{
+    Sample<2> s;
+    const float d0 = k.c[1] - k.c[0], d1 = k.c[3] - k.c[2];
+    const float v0 = fmaf(k.tx, d0, k.c[0]), v1 = fmaf(k.tx, d1, k.c[2]);
+    const float gy = v1 - v0;
+    s.val = fmaf(k.ty, gy, v0);
+    if (WANT_GRAD) {
+        s.g[1] = gy;
+        s.g[0] = fmaf(k.ty, d1 - d0, d0);
+    }
+    return s;
+}
+
 // Value at a second position that usually lies in the cell already gathered (a gradient step moves a sample by a
 // fraction of a voxel): same corners, new fractions — bit-identical to a fresh gather, without its 8 loads.
 __device__ __forceinline__ float sample_near(const Cell3 &k, const float *__restrict__ m, int D, int H, int W,
@@ -203,27 +240,12 @@ __device__ __forceinline__ Sample<NDIM> sample_zero_pad(const float *__restrict_
     if constexpr (NDIM == 3) {
         return blend_cell3<WANT_GRAD>(gather_cell3<BRANCH_FREE>(m, D, H, W, px, py, pz));
     } else {
-        Sample<NDIM> s;
+        Cell2 k;
         int x0, y0;
-        float tx, ty;
-        floor_frac(px, x0, tx);
-        floor_frac(py, y0, ty);
-        const bool vx0 = (unsigned)x0 < (unsigned)W, vx1 = (unsigned)(x0 + 1) < (unsigned)W;
-        const bool vy0 = (unsigned)y0 < (unsigned)H, vy1 = (unsigned)(y0 + 1) < (unsigned)H;
-        const float *q = m + ((long long)y0 * W + x0);
-        const float c00 = (vy0 & vx0) ? __ldg(q) : 0.f;
-        const float c01 = (vy0 & vx1) ? __ldg(q + 1) : 0.f;
-        const float c10 = (vy1 & vx0) ? __ldg(q + W) : 0.f;
-        const float c11 = (vy1 & vx1) ? __ldg(q + W + 1) : 0.f;
-        const float d0 = c01 - c00, d1 = c11 - c10;
-        const float v0 = fmaf(tx, d0, c00), v1 = fmaf(tx, d1, c10);
-        const float gy = v1 - v0;
-        s.val = fmaf(ty, gy, v0);
-        if (WANT_GRAD) {
-            s.g[1] = gy;
-            s.g[0] = fmaf(ty, d1 - d0, d0);
-        }
-        return s;
+        floor_frac(px, x0, k.tx);
+        floor_frac(py, y0, k.ty);
+        load_cell2(m, H, W, x0, y0, k.c);
+        return blend_cell2<WANT_GRAD>(k);
     }
 }
 

@@ -33,52 +33,6 @@ struct WarpParams {
     int n_channels;
 };
 
-// value of two voxels (z, z+1) from the staged box: the interpolation half of pair_step
-template <int BX, int BY>
-__device__ __forceinline__ float2 pair_value(uint32_t box_m, float Mrel, float2 ix, float2 iy, float2 iz)
-{
-    const float2 M = f2(kMagic), nM = f2(-kMagic);
-    const float2 flx = __fadd2_rd(ix, M), fly = __fadd2_rd(iy, M), flz = __fadd2_rd(iz, M);
-    const float2 fx = __fadd2_rn(flx, nM), fy = __fadd2_rn(fly, nM), fz = __fadd2_rn(flz, nM);
-    const float2 tx = sub2(ix, fx), ty = sub2(iy, fy), tz = sub2(iz, fz);
-    const float2 tb = __ffma2_rn(f2(kIdxScale * (float)(BX * BY)), fz,
-                                 __ffma2_rn(f2(kIdxScale * (float)BX), fy, __ffma2_rn(f2(kIdxScale), fx, f2(Mrel))));
-    const uint32_t qa = box_m + ((uint32_t)__float_as_int(tb.x) << 2);
-    const uint32_t qb = box_m + ((uint32_t)__float_as_int(tb.y) << 2);
-    constexpr int SY = BX * 4, SZ = BX * BY * 4;
-    const float2 c000 = make_float2(lds_f<0>(qa), lds_f<0>(qb)), c001 = make_float2(lds_f<4>(qa), lds_f<4>(qb));
-    const float2 c010 = make_float2(lds_f<SY>(qa), lds_f<SY>(qb)), c011 = make_float2(lds_f<SY + 4>(qa), lds_f<SY + 4>(qb));
-    const float2 c100 = make_float2(lds_f<SZ>(qa), lds_f<SZ>(qb)), c101 = make_float2(lds_f<SZ + 4>(qa), lds_f<SZ + 4>(qb));
-    const float2 c110 = make_float2(lds_f<SZ + SY>(qa), lds_f<SZ + SY>(qb));
-    const float2 c111 = make_float2(lds_f<SZ + SY + 4>(qa), lds_f<SZ + SY + 4>(qb));
-    const float2 v00 = __ffma2_rn(tx, sub2(c001, c000), c000), v01 = __ffma2_rn(tx, sub2(c011, c010), c010);
-    const float2 v10 = __ffma2_rn(tx, sub2(c101, c100), c100), v11 = __ffma2_rn(tx, sub2(c111, c110), c110);
-    const float2 w0 = __ffma2_rn(ty, sub2(v01, v00), v00), w1 = __ffma2_rn(ty, sub2(v11, v10), v10);
-    return __ffma2_rn(tz, sub2(w1, w0), w0);
-}
-
-__device__ __forceinline__ float value_direct(const float *__restrict__ mov, int D, int H, int W, float ix, float iy, float iz)
-{
-    ix = fminf(fmaxf(ix, -4.f), (float)W + 4.f);
-    iy = fminf(fmaxf(iy, -4.f), (float)H + 4.f);
-    iz = fminf(fmaxf(iz, -4.f), (float)D + 4.f);
-    const float fx = __fadd_rd(ix, kMagic) - kMagic, fy = __fadd_rd(iy, kMagic) - kMagic, fz = __fadd_rd(iz, kMagic) - kMagic;
-    const float tx = ix - fx, ty = iy - fy, tz = iz - fz;
-    const int x0 = (int)fx, y0 = (int)fy, z0 = (int)fz;
-    const bool vx0 = (unsigned)x0 < (unsigned)W, vx1 = (unsigned)(x0 + 1) < (unsigned)W;
-    const bool vy0 = (unsigned)y0 < (unsigned)H, vy1 = (unsigned)(y0 + 1) < (unsigned)H;
-    const bool vz0 = (unsigned)z0 < (unsigned)D, vz1 = (unsigned)(z0 + 1) < (unsigned)D;
-    const long long HW = (long long)H * W, o = ((long long)z0 * H + y0) * W + x0;
-    const float c000 = (vz0 & vy0 & vx0) ? __ldg(mov + o) : 0.f, c001 = (vz0 & vy0 & vx1) ? __ldg(mov + o + 1) : 0.f;
-    const float c010 = (vz0 & vy1 & vx0) ? __ldg(mov + o + W) : 0.f, c011 = (vz0 & vy1 & vx1) ? __ldg(mov + o + W + 1) : 0.f;
-    const float c100 = (vz1 & vy0 & vx0) ? __ldg(mov + o + HW) : 0.f, c101 = (vz1 & vy0 & vx1) ? __ldg(mov + o + HW + 1) : 0.f;
-    const float c110 = (vz1 & vy1 & vx0) ? __ldg(mov + o + HW + W) : 0.f, c111 = (vz1 & vy1 & vx1) ? __ldg(mov + o + HW + W + 1) : 0.f;
-    const float v00 = fmaf(tx, c001 - c000, c000), v01 = fmaf(tx, c011 - c010, c010);
-    const float v10 = fmaf(tx, c101 - c100, c100), v11 = fmaf(tx, c111 - c110, c110);
-    const float w0 = fmaf(ty, v01 - v00, v00), w1 = fmaf(ty, v11 - v10, v10);
-    return fmaf(tz, w1 - w0, w0);
-}
-
 __global__ void __launch_bounds__(kWarpThreads, 1)
 warp_affine_tma_kernel(const WarpParams wp, const __grid_constant__ CUtensorMap map_mov)
 {
@@ -224,7 +178,7 @@ warp_affine_tma_kernel(const WarpParams wp, const __grid_constant__ CUtensorMap 
                     const float2 ix = __ffma2_rn(f2(sz[0]), zf, f2(pxy[0]));
                     const float2 iy = __ffma2_rn(f2(sz[1]), zf, f2(pxy[1]));
                     const float2 iz = __ffma2_rn(f2(sz[2]), zf, f2(pxy[2]));
-                    const float2 v = pair_value<kBX, kBY>(box_addr, m.Mrel, ix, iy, iz);
+                    const float2 v = pair_sample<kBX, kBY, false>(box_addr, box_cells<kBX, kBY>(m.Mrel, ix, iy, iz)).val;
                     __stcs(o + (size_t)(2 * j) * HW, v.x);
                     __stcs(o + (size_t)(2 * j + 1) * HW, v.y);
                     zf = __fadd2_rn(zf, f2(2.f));
@@ -233,14 +187,16 @@ warp_affine_tma_kernel(const WarpParams wp, const __grid_constant__ CUtensorMap 
                 for (int zz = 0; zz < m.nz; ++zz) {
                     const float za = m.zf0 + (float)zz;
                     const float2 zf = make_float2(za, za);
-                    const float2 v = pair_value<kBX, kBY>(box_addr, m.Mrel, __ffma2_rn(f2(sz[0]), zf, f2(pxy[0])),
-                                                          __ffma2_rn(f2(sz[1]), zf, f2(pxy[1])), __ffma2_rn(f2(sz[2]), zf, f2(pxy[2])));
+                    const BoxCells c = box_cells<kBX, kBY>(m.Mrel, __ffma2_rn(f2(sz[0]), zf, f2(pxy[0])),
+                                                           __ffma2_rn(f2(sz[1]), zf, f2(pxy[1])), __ffma2_rn(f2(sz[2]), zf, f2(pxy[2])));
+                    const float2 v = pair_sample<kBX, kBY, false>(box_addr, c).val;
                     __stcs(o + (size_t)zz * HW, v.x);
                 }
             } else {
                 for (int zz = 0; zz < m.nz; ++zz) {
                     const float zf = m.zf0 + (float)zz;
-                    __stcs(o + (size_t)zz * HW, value_direct(mov, D, H, W, fmaf(sz[0], zf, pxy[0]), fmaf(sz[1], zf, pxy[1]), fmaf(sz[2], zf, pxy[2])));
+                    const Cell3 k = gather_clamped3(mov, D, H, W, fmaf(sz[0], zf, pxy[0]), fmaf(sz[1], zf, pxy[1]), fmaf(sz[2], zf, pxy[2]));
+                    __stcs(o + (size_t)zz * HW, blend_cell3<false>(k).val);
                 }
             }
         }
