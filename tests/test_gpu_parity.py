@@ -1288,3 +1288,97 @@ def test_fused_unet_head_equals_unfused_path(shape, weights):
         num += ((d_got - d_ref) ** 2).sum().item()
         den += (d_ref ** 2).sum().item()
     assert (num / max(den, 1e-300)) ** 0.5 <= 2e-3, "parameter step: relative L2 difference %.2e" % ((num / max(den, 1e-300)) ** 0.5)
+
+
+def test_fixed_order_reductions_are_bit_reproducible():
+    """The fp64 block / grid reductions (common.cuh: block_sum, grid_sum, last_to_arrive) promise the same bits on
+    every run.  Each family is called at shape A, then at a shape B with a different grid size, then at A again: the two
+    A results must be identical.  A ticket that is not re-armed, or a fold whose order depends on timing, breaks this."""
+    TF = _tf()
+    from torchregister_b200.synth import make_pair, smooth_flow
+
+    def same_after_other_grid(run, a, b):
+        first = [t.clone() for t in run(a)]
+        run(b)
+        again = run(a)
+        for x, y in zip(first, again):
+            assert torch.equal(x, y)
+
+    def seeded(shape, seed, n=1, scale=1.0):
+        g = torch.Generator(device="cpu").manual_seed(seed)
+        return (scale * torch.randn((n,) + tuple(shape), generator=g)).to(DEV)
+
+    pairs = {s: tuple(t.to(DEV) for t in make_pair(s, "flow")) for s in [(24, 20, 16), (40, 36, 44), (48, 40), (96, 72)]}
+
+    def flow_node(shape, w_ncc):
+        mov, tgt = pairs[shape]
+        flow = 0.5 * smooth_flow(shape, 1.0).to(DEV)
+        loss, dflow, warped = TF.flow_loss_grad(mov, tgt, flow, 0.5, w_ncc, want_warped=True)
+        return loss, dflow, warped
+
+    for w_ncc in (0.0, 0.5):
+        same_after_other_grid(lambda s: flow_node(s, w_ncc), (24, 20, 16), (40, 36, 44))
+
+    def head(shape):
+        mov, tgt = pairs[shape]
+        nd = len(shape)
+        feat = seeded((3,) + tuple(v - 2 for v in shape), 5)
+        w, b = seeded((nd, 3) + (1,) * nd, 6, n=1)[0], seeded((nd,), 7, n=1)[0]
+        loss, flow = TF.flow_head_forward(mov, tgt, feat, w, b, 0.5, 0.5)
+        dfeat, dw, db = TF.flow_head_backward(mov, tgt, flow, feat, w)
+        return loss, flow, dfeat, dw, db
+
+    same_after_other_grid(head, (24, 20, 16), (40, 36, 44))
+    same_after_other_grid(head, (48, 40), (96, 72))
+
+    def direct(shape, opt, weights, smooth, two_pass):
+        mov, tgt = (t.to(DEV) for t in make_pair(shape, "flow"))
+        p = TF.DirectFlowProblem(mov, tgt, 3, flow0=(0.3 * smooth_flow(shape, 1.0)).to(DEV), optimiser=opt)
+        lr = 0.5 if opt == "sgd" else 0.05
+        (p.run_two_pass if two_pass else p.run)(3, lr, weights[0], weights[1], smooth)
+        return p.flow, p.losses
+
+    same_after_other_grid(lambda s: direct(s, "sgd", (0.5, 0.5), 4.0, True), (48, 40), (96, 72))
+    same_after_other_grid(lambda s: direct(s, "adam", (0.5, 0.5), 4.0, True), (13, 19, 37), (21, 33, 72))
+    # fused epoch: register-staged kernel (no smoothing, or W % 4 != 0) and TMA-staged kernel (smoothing, W % 4 == 0)
+    for opt in ("sgd", "adam"):
+        for weights in ((1.0, 0.0), (0.5, 0.5)):
+            same_after_other_grid(lambda s: direct(s, opt, weights, 0.0, False), (13, 19, 37), (40, 33, 70))
+            same_after_other_grid(lambda s: direct(s, opt, weights, 4.0, False), (12, 16, 40), (21, 33, 72))
+
+    def convs(shape):
+        x = seeded((2,) + shape, 8)
+        w3, gy3 = seeded((2, 2, 3, 3, 3), 9)[0], seeded((2,) + tuple(v - 2 for v in shape), 10)
+        w1, gy1 = seeded((2, 2, 1, 1, 1), 11)[0], seeded((2,) + shape, 12)
+        wu, gyu = seeded((2, 2, 2, 2, 2), 13)[0], seeded((2,) + tuple(2 * v for v in shape), 14)
+        out = []
+        for r in (TF.thin_conv3d_backward(x, w3, gy3, True, True, True), TF.point_conv3d_backward(x, w1, gy1, 1, True, True, True),
+                  TF.up_conv3d_backward(x, wu, gyu, True, True, True)):
+            out += list(r)
+        return out
+
+    same_after_other_grid(convs, (12, 14, 40), (30, 33, 70))
+
+    def instnorm(shape):
+        x, dy = seeded((3,) + shape, 15), seeded((3,) + shape, 16)
+        gate = seeded((1,) + shape, 17).sigmoid()
+        y, st = TF.instance_norm_forward(x, relu=True)
+        dx = TF.instance_norm_backward(x, dy, st, relu=True)
+        yg, stg = TF.instance_norm_forward(x, gate=gate)
+        dxg, dgate = TF.instance_norm_backward(x, dy, stg, gate=gate)
+        return y, st, dx, yg, stg, dxg, dgate
+
+    same_after_other_grid(instnorm, (20, 22, 40), (64, 60, 66))
+
+    nmi_terms = {}
+
+    def nmi(shape):
+        mov, tgt = (t.to(DEV) for t in make_pair(shape, "rigid"))
+        if shape not in nmi_terms:
+            lo, hi = TF.NmiSourceTerm.bounds(mov, tgt)
+            nmi_terms[shape] = (TF.NmiTerm(tgt * 255.0), TF.NmiTerm(tgt), TF.NmiSourceTerm(tgt, lo, hi))
+        res, src = nmi_terms[shape][:2], nmi_terms[shape][2]
+        return [v.clone() for t, s in zip(res, (255.0, 1.0)) for v in t.loss_grad(mov * s, 1.0)] + list(src.loss_grad(mov, 1.0))
+
+    same_after_other_grid(nmi, (24, 32, 40), (40, 47, 33))
+    same_after_other_grid(nmi, (64, 48), (300, 180))

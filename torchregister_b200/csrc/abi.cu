@@ -22,6 +22,20 @@ int check_cuda(cudaError_t e, const char *what)
     return (int)e;
 }
 
+// grid sizes follow the SM count; launchers ask on every call, so the answer is cached per device ordinal
+static int g_sm_count[64] = {};
+
+int sm_count(int &n)
+{
+    int dev = 0;
+    int rc = check_cuda(cudaGetDevice(&dev), "cudaGetDevice");
+    if (rc) return rc;
+    int &c = g_sm_count[dev & 63];
+    if (c == 0) rc = check_cuda(cudaDeviceGetAttribute(&c, cudaDevAttrMultiProcessorCount, dev), "SM count");
+    n = c;
+    return rc;
+}
+
 }  // namespace trb
 
 extern "C" int trb_abi_version(void) { return TRB_ABI_VERSION; }

@@ -287,16 +287,7 @@ __global__ void affine_set_params_kernel(float *state, int n, int n_params, cons
 }
 
 // ---- host side ---------------------------------------------------------------------------
-static int g_sm_count[64] = {};       // per device ordinal
 static bool g_force_direct = false;   // test hook: trb_set_kernel_path(1) pins the non-TMA kernel
-static int sm_count()
-{
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return -1;
-    int &n = g_sm_count[dev & 63];
-    if (n == 0 && cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return -1;
-    return n;
-}
 
 constexpr int kMaxBlocksPerPair = kMaxSlots;
 
@@ -305,9 +296,8 @@ static size_t affine_ws_bytes(int n_pairs)
     return (size_t)n_pairs * kMaxBlocksPerPair * TRB_MOMENTS * sizeof(double) + (size_t)n_pairs * kTicketStride * sizeof(unsigned);
 }
 
-static int blocks_per_pair(int rows, int n_pairs)
+static int blocks_per_pair(int rows, int n_pairs, int sms)
 {
-    const int sms = sm_count();
     const int groups = (rows + kWarps - 1) / kWarps;
     // two resident CTAs per SM; whole waves across the batch
     int per = (2 * sms + n_pairs - 1) / n_pairs;
@@ -321,7 +311,11 @@ static int blocks_per_pair(int rows, int n_pairs)
 
 using namespace trb;
 
-extern "C" int trb_sm_count(void) { return sm_count(); }
+extern "C" int trb_sm_count(void)
+{
+    int n = 0;
+    return sm_count(n) ? -1 : n;
+}
 
 extern "C" int trb_set_kernel_path(int path)
 {
@@ -518,8 +512,10 @@ extern "C" int trb_affine_optim_ex(int ndim, int mode, const float *moving_dev, 
         if (rc != TRB_ERR_UNSUPPORTED) return rc;
         return launch_affine3d_tma(p, n_pairs, true, epoch0, n_epochs, s);  // one launch per epoch
     }
+    int sms;
+    if ((rc = sm_count(sms))) return rc;
     const int rows = ndim == 3 ? D * H : H;
-    const dim3 grid(blocks_per_pair(rows, n_pairs), n_pairs);
+    const dim3 grid(blocks_per_pair(rows, n_pairs, sms), n_pairs);
     for (int e = 0; e < n_epochs; ++e) {
         p.epoch = epoch0 + e;
         if (ndim == 3) affine_moments_kernel<3, true><<<grid, kThreads, 0, s>>>(p);
@@ -581,6 +577,8 @@ int trb::affine_moments_impl(int ndim, const float *moving_dev, const float *tar
     p.state = const_cast<float *>(state_dev);
     p.moments_out = moments_dev;
     p.gather = (flags & TRB_FLAG_LARGE_ROTATION) ? ((flags & TRB_FLAG_QUAD_VOLUME) ? 3 : (flags & TRB_FLAG_PAIR_VOLUME) ? 2 : 1) : 0;
+    int sms;
+    if ((rc = sm_count(sms))) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     if (!g_force_direct && tma_path_eligible(ndim, p, n_pairs)) {
         // both TMA-tile kernels store the warped samples on request (whole volumes of single-channel pairs only)
@@ -591,7 +589,7 @@ int trb::affine_moments_impl(int ndim, const float *moving_dev, const float *tar
         // pass would have to recompute the target sums (a separate pass over the targets in the persistent design: the
         // default-loss loop caches them after its first epoch, a stand-alone trb_affine_moments call cannot)
         const long long tiles = (long long)n_pairs * ((W + TX - 1) / TX) * ((H + TY - 1) / TY) * ((s_end - s_begin + TZ - 1) / TZ);
-        if (p.gather || (target_sums != 1 && tiles >= 10LL * sm_count())) {
+        if (p.gather || (target_sums != 1 && tiles >= 10LL * sms)) {
             if (store) p.warped_out = warped_out;
             rc = launch_affine3d_persist(p, n_pairs, 0, 1, s, target_sums == 0 ? 2 : (target_sums == 2 ? 3 : 1));   // 1 and 3: compute
             if (rc != TRB_ERR_UNSUPPORTED) {
@@ -607,7 +605,7 @@ int trb::affine_moments_impl(int ndim, const float *moving_dev, const float *tar
         return launch_affine3d_tma(p, n_pairs, false, 0, 1, s);
     }
     const int rows = (s_end - s_begin) * (ndim == 3 ? H : 1);
-    const dim3 grid(blocks_per_pair(rows, n_pairs), n_pairs);
+    const dim3 grid(blocks_per_pair(rows, n_pairs, sms), n_pairs);
     if (ndim == 3) affine_moments_kernel<3, false><<<grid, kThreads, 0, s>>>(p);
     else affine_moments_kernel<2, false><<<grid, kThreads, 0, s>>>(p);
     return check_cuda(cudaGetLastError(), "affine_moments");
@@ -680,7 +678,8 @@ extern "C" int trb_warp_affine_batch(int ndim, const float *moving_dev, float *o
     if (ndim == 3 && !g_force_direct && !(flags & TRB_FLAG_LARGE_ROTATION) &&
         warp_tma_eligible(moving_dev, out_dev, n_pairs * n_channels, (long long)vol, D, H, W))
         return launch_warp_affine_tma(moving_dev, out_dev, n_pairs, n_channels, D, H, W, theta_dev, xb_dev, yb_dev, s);
-    const int sms = sm_count();
+    int sms;
+    if ((rc = sm_count(sms))) return rc;
     size_t nb = (vol + 255) / 256;
     if (nb > (size_t)sms * 16) nb = (size_t)sms * 16;
     const dim3 grid((unsigned)nb, (unsigned)n_pairs);

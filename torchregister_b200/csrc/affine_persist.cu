@@ -888,10 +888,10 @@ int launch_affine3d_persist(AffineParams a, int n_pairs, int epoch0, int n_epoch
     if (g_no_persist || a.extra) PERSIST_REFUSE("disabled (kernel path / extra term)");
     if (a.peer.world > 1 && n_pairs != 1) PERSIST_REFUSE("peer exchange needs one pair");
     int dev = 0, sms = 0, coop = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) PERSIST_REFUSE("cudaGetDevice failed");
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (int rc = sm_count(sms)) return rc;
+    cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
-    if (!coop || sms < 1) PERSIST_REFUSE("no cooperative launch (coop %d, sms %d)", coop, sms);
+    if (!coop) PERSIST_REFUSE("no cooperative launch");
     const bool mse_only = !moments_only && a.w_ncc == 0.f;
     const bool rot = a.gather != 0;
     const bool store = moments_only && !rot && a.warped_out != nullptr;

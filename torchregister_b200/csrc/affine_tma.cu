@@ -495,9 +495,9 @@ int launch_affine3d_tma(AffineParams a, int n_pairs, bool fused, int epoch0, int
     p.tiles_x = (a.W + TX - 1) / TX;
     p.tiles_y = (a.H + TY - 1) / TY;
     p.tiles_z = (a.s_end - a.s_begin + TZ - 1) / TZ;
-    int dev = 0, sms = 148;
+    int sms, dev = 0;
+    if ((rc = sm_count(sms))) return rc;
     cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     p.cols_per_pair = p.tiles_x * p.tiles_y;
     const long long total_cols = (long long)n_pairs * p.cols_per_pair;
     long long grid_ll = sms;

@@ -16,6 +16,8 @@ constexpr unsigned kFull = 0xffffffffu;
 
 void set_error(const char *fmt, ...);
 int check_cuda(cudaError_t e, const char *what);
+// SM count of the current device, queried once per device.  Returns TRB_OK, or the CUDA error with trb_last_error() set.
+int sm_count(int &n);
 
 // ---- loads ---------------------------------------------------------------
 __device__ __forceinline__ float ldg_f(const float *p) { return __ldg(p); }
@@ -39,6 +41,101 @@ __device__ __forceinline__ double warp_sum(double v)
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(kFull, v, o);
     return v;
+}
+
+// ---- fixed-order (deterministic) block and grid reductions of fp64 sums, for 256-thread CTAs ----------------------
+// Every sum is formed in the same order on every run: the warp_sum shuffle tree, then warps 0..7 in order, then the
+// blocks in index order.  The caller declares the shared rows, so each kernel's footprint stays visible.
+
+// Block total of each entry: thread i < N returns the total of v[i] (fp32 inputs are widened first), others 0.
+template <int N, typename T>
+__device__ __forceinline__ double block_sum(const T (&v)[N], double (&sh)[kWarps][N])
+{
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int i = 0; i < N; ++i) {
+        const double s = warp_sum((double)v[i]);
+        if (lane == 0) sh[warp][i] = s;
+    }
+    __syncthreads();
+    double t = 0.0;
+    if (threadIdx.x < N) {
+#pragma unroll
+        for (int w = 0; w < kWarps; ++w) t += sh[w][threadIdx.x];
+    }
+    return t;
+}
+
+// The same order, but every thread gets all N totals in v.  Starts with a barrier, so consecutive calls can share sh
+// (any M >= N columns).
+template <int N, int M>
+__device__ __forceinline__ void block_sum_all(double (&v)[N], double (&sh)[kWarps][M])
+{
+    static_assert(N <= M, "shared rows too short");
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int i = 0; i < N; ++i) v[i] = warp_sum(v[i]);
+    __syncthreads();
+    if (lane == 0) {
+#pragma unroll
+        for (int i = 0; i < N; ++i) sh[warp][i] = v[i];
+    }
+    __syncthreads();
+#pragma unroll
+    for (int i = 0; i < N; ++i) {
+        double t = 0.0;
+#pragma unroll
+        for (int w = 0; w < kWarps; ++w) t += sh[w][i];
+        v[i] = t;
+    }
+}
+template <int M>
+__device__ __forceinline__ double block_sum_all(double v, double (&sh)[kWarps][M])
+{
+    double a[1] = {v};
+    block_sum_all(a, sh);
+    return a[0];
+}
+
+// Called by every thread of a block after it has stored its share of a grid-wide result.  True, in every thread, for
+// the block that arrives last of `expected`; that block then sees what the others stored.  The fences pair the others'
+// stores with this block's loads; the caller re-arms the ticket (*ticket = 0) once it is done.
+__device__ __forceinline__ bool last_to_arrive(unsigned *ticket, unsigned expected)
+{
+    __threadfence();
+    __syncthreads();
+    int last = 0;
+    if (threadIdx.x == 0) last = atomicAdd(ticket, 1u) == expected - 1;
+    last = __syncthreads_or(last);
+    if (last) __threadfence();
+    return last;
+}
+
+// One warp: sum over blocks 0..n_blocks-1 of part[b * stride + k], lane l taking blocks l, l+32, ... then warp_sum.
+__device__ __forceinline__ double fold_blocks(const double *part, int n_blocks, size_t stride, int k)
+{
+    double t = 0.0;
+    for (int b = threadIdx.x & 31; b < n_blocks; b += 32) t += __ldcg(part + (size_t)b * stride + k);
+    return warp_sum(t);
+}
+
+// Grid total of each entry: the block totals go to partials[block][N], and the last block to arrive adds them in block
+// order into sh[0][0..N) and re-arms the ticket.  Returns true in every thread of that block (sh is then ready), false
+// in the others.
+template <int N, typename T>
+__device__ __forceinline__ bool grid_sum(const T (&v)[N], double (&sh)[kWarps][N], double *partials, unsigned *ticket)
+{
+    const double t = block_sum(v, sh);
+    if (threadIdx.x < N) __stcg(partials + (size_t)blockIdx.x * N + threadIdx.x, t);
+    if (!last_to_arrive(ticket, gridDim.x)) return false;
+    const int warp = threadIdx.x >> 5;
+    for (int i = warp; i < N; i += kWarps) {
+        const double s = fold_blocks(partials, gridDim.x, N, i);
+        if ((threadIdx.x & 31) == 0) sh[0][i] = s;
+    }
+    if (threadIdx.x == 0) *ticket = 0u;
+    __syncthreads();
+    return true;
 }
 
 // Row-wise voxel loop: a 256-thread CTA takes two rows (z,y) at a time, 128 threads along x each, so the only

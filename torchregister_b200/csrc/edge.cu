@@ -93,9 +93,8 @@ extern "C" int trb_edge3d(const float *img_dev, float *out_dev, int B, int C, in
     e = cudaMemcpyAsync(minmax_dev, init, sizeof(init), cudaMemcpyHostToDevice, s);
     if (e != cudaSuccess) return check_cuda(e, "cudaMemcpyAsync(minmax)");
     const size_t total = (size_t)B * X * Y * Z;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    int sms;
+    if (int rc = sm_count(sms)) return rc;
     size_t nb = (total + 255) / 256;
     if (nb > (size_t)sms * 8) nb = (size_t)sms * 8;
     edge_grad_kernel<<<(unsigned)nb, 256, 0, s>>>(img_dev, out_dev, B, C, X, Y, Z, minmax_dev);

@@ -100,46 +100,11 @@ __global__ void __launch_bounds__(256) flow_stats_kernel(const float *__restrict
         s[0] += t; s[1] += w;
         s[2] = fmaf(t, t, s[2]); s[3] = fmaf(w, w, s[3]); s[4] = fmaf(t, w, s[4]);
     });
-    double acc[5];
-#pragma unroll
-    for (int i = 0; i < 5; ++i) acc[i] = (double)s[i];
-    __shared__ double red[8][5];
-    __shared__ bool is_last;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-    for (int i = 0; i < 5; ++i) {
-        const double v = warp_sum(acc[i]);
-        if (lane == 0) red[warp][i] = v;
-    }
-    __syncthreads();
-    double *partials = ws + 8;
-    unsigned *ticket = (unsigned *)(ws + 4);
-    if (threadIdx.x < 5) {
-        double v = 0.0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) v += red[w][threadIdx.x];
-        __stcg(partials + (size_t)blockIdx.x * 5 + threadIdx.x, v);
-    }
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) is_last = (atomicAdd(ticket, 1u) == gridDim.x - 1);
-    __syncthreads();
-    if (!is_last) return;
-    __threadfence();
-    // fixed-order reduction over blocks: warp i < 5 sums moment i
-    if (warp < 5) {
-        double v = 0.0;
-        for (int b = lane; b < (int)gridDim.x; b += 32) v += __ldcg(partials + (size_t)b * 5 + warp);
-        v = warp_sum(v);
-        if (lane == 0) red[0][warp] = v;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const LossCoef lc = loss_coefficients((double)vol, red[0][0], red[0][1], red[0][2], red[0][3], red[0][4], w_mse, w_ncc);
-        ws[0] = lc.cw; ws[1] = lc.ct; ws[2] = lc.c0; ws[3] = lc.loss;
-        if (loss_out) *loss_out = (float)lc.loss;
-        *ticket = 0u;
-    }
+    __shared__ double red[kWarps][5];
+    if (!grid_sum(s, red, ws + 8, (unsigned *)(ws + 4)) || threadIdx.x != 0) return;
+    const LossCoef lc = loss_coefficients((double)vol, red[0][0], red[0][1], red[0][2], red[0][3], red[0][4], w_mse, w_ncc);
+    ws[0] = lc.cw; ws[1] = lc.ct; ws[2] = lc.c0; ws[3] = lc.loss;
+    if (loss_out) *loss_out = (float)lc.loss;
 }
 
 template <int NDIM>
@@ -171,7 +136,7 @@ __global__ void __launch_bounds__(256) flow_mse_fused_kernel(const float *__rest
     const size_t vol = (size_t)(NDIM == 3 ? D : 1) * H * W;
     const FlowAxes ax = flow_axes(D, H, W);
     const float gm = (float)(2.0 * w_mse / (double)vol);
-    float sd = 0.f;
+    float sd[1] = {0.f};
     for_each_voxel(NDIM == 3 ? D : 1, H, W, [&](size_t idx, int x, int y, int z) {
         float px, py, pz;
         flow_position<NDIM>(flow, vol, idx, x, y, z, ax, px, py, pz);
@@ -179,39 +144,14 @@ __global__ void __launch_bounds__(256) flow_mse_fused_kernel(const float *__rest
         const float t = ld_stream_f(target + idx);
         const float d = s.val - t;
         if (warped) warped[idx] = s.val;
-        sd = fmaf(d, d, sd);
+        sd[0] = fmaf(d, d, sd[0]);
         store_dflow<NDIM>(dflow, vol, idx, gm * d, s.g);
     });
-    __shared__ double red[8];
-    __shared__ bool is_last;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const double v = warp_sum((double)sd);
-    if (lane == 0) red[warp] = v;
-    __syncthreads();
-    double *partials = ws + 8;
-    unsigned *ticket = (unsigned *)(ws + 4);
-    if (threadIdx.x == 0) {
-        double t = 0.0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) t += red[w];
-        __stcg(partials + blockIdx.x, t);
-        __threadfence();
-        is_last = (atomicAdd(ticket, 1u) == gridDim.x - 1);
-    }
-    __syncthreads();
-    if (!is_last) return;
-    __threadfence();
-    if (warp == 0) {                               // fixed-order reduction over blocks
-        double t = 0.0;
-        for (int b = lane; b < (int)gridDim.x; b += 32) t += __ldcg(partials + b);
-        t = warp_sum(t);
-        if (lane == 0) {
-            const double loss = w_mse * t / (double)vol;
-            ws[3] = loss;
-            if (loss_out) *loss_out = (float)loss;
-            *ticket = 0u;
-        }
-    }
+    __shared__ double red[kWarps][1];
+    if (!grid_sum(sd, red, ws + 8, (unsigned *)(ws + 4)) || threadIdx.x != 0) return;
+    const double loss = w_mse * red[0][0] / (double)vol;
+    ws[3] = loss;
+    if (loss_out) *loss_out = (float)loss;
 }
 
 // ---- U-Net head fused with the node (SURVEY.md §8 f-3; reference utils.py:553-557) ---------------------------------
@@ -279,42 +219,11 @@ __global__ void __launch_bounds__(256) flow_head_forward_kernel(const float *__r
         s[0] += t; s[1] += w;
         s[2] = fmaf(t, t, s[2]); s[3] = fmaf(w, w, s[3]); s[4] = fmaf(t, w, s[4]);
     });
-    __shared__ double red[8][5];
-    __shared__ bool is_last;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-    for (int i = 0; i < 5; ++i) {
-        const double v = warp_sum((double)s[i]);
-        if (lane == 0) red[warp][i] = v;
-    }
-    __syncthreads();
-    double *partials = ws + 8;
-    unsigned *ticket = (unsigned *)(ws + 4);
-    if (threadIdx.x < 5) {
-        double v = 0.0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) v += red[w][threadIdx.x];
-        __stcg(partials + (size_t)blockIdx.x * 5 + threadIdx.x, v);
-    }
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) is_last = (atomicAdd(ticket, 1u) == gridDim.x - 1);
-    __syncthreads();
-    if (!is_last) return;
-    __threadfence();
-    if (warp < 5) {
-        double v = 0.0;
-        for (int b = lane; b < (int)gridDim.x; b += 32) v += __ldcg(partials + (size_t)b * 5 + warp);
-        v = warp_sum(v);
-        if (lane == 0) red[0][warp] = v;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const LossCoef lc = loss_coefficients((double)vol, red[0][0], red[0][1], red[0][2], red[0][3], red[0][4], w_mse, w_ncc);
-        ws[0] = lc.cw; ws[1] = lc.ct; ws[2] = lc.c0; ws[3] = lc.loss;
-        if (loss_out) *loss_out = (float)lc.loss;
-        *ticket = 0u;
-    }
+    __shared__ double red[kWarps][5];
+    if (!grid_sum(s, red, ws + 8, (unsigned *)(ws + 4)) || threadIdx.x != 0) return;
+    const LossCoef lc = loss_coefficients((double)vol, red[0][0], red[0][1], red[0][2], red[0][3], red[0][4], w_mse, w_ncc);
+    ws[0] = lc.cw; ws[1] = lc.ct; ws[2] = lc.c0; ws[3] = lc.loss;
+    if (loss_out) *loss_out = (float)lc.loss;
 }
 
 // d loss / d flow (registers) -> d feat [C][fd][fh][fw], d W [ndim][C], d b [ndim] (dwb_out: ndim*(C+1) floats, W first)
@@ -360,53 +269,24 @@ __global__ void __launch_bounds__(256) flow_head_backward_kernel(const float *__
             }
         }
     });
-    __shared__ double red[8][NS];
-    __shared__ bool is_last;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-    for (int i = 0; i < NS; ++i) {
-        const double v = warp_sum((double)acc[i]);
-        if (lane == 0) red[warp][i] = v;
-    }
-    __syncthreads();
-    double *partials = ws + 8;                       // [blocks][NS]  (the forward pass is done with the 5-wide rows)
-    unsigned *ticket = (unsigned *)(ws + 4);
-    if (threadIdx.x < NS) {
-        double v = 0.0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) v += red[w][threadIdx.x];
-        __stcg(partials + (size_t)blockIdx.x * NS + threadIdx.x, v);
-    }
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) is_last = (atomicAdd(ticket, 1u) == gridDim.x - 1);
-    __syncthreads();
-    if (!is_last) return;
-    __threadfence();
-    for (int i = warp; i < NS; i += 8) {             // fixed-order reduction over blocks
-        double v = 0.0;
-        for (int b = lane; b < (int)gridDim.x; b += 32) v += __ldcg(partials + (size_t)b * NS + i);
-        v = warp_sum(v);
-        if (lane == 0) {
-            const int a = i / (kHeadMaxC + 1), c = i - a * (kHeadMaxC + 1);
-            if (c < h.C) dwb_out[a * h.C + c] = (float)v;
-            else if (c == kHeadMaxC) dwb_out[NDIM * h.C + a] = (float)v;
-        }
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) *ticket = 0u;
+    // partials [blocks][NS]: the forward pass is done with the 5-wide rows
+    __shared__ double red[kWarps][NS];
+    if (!grid_sum(acc, red, ws + 8, (unsigned *)(ws + 4)) || threadIdx.x >= NS) return;
+    const int i = threadIdx.x, a = i / (kHeadMaxC + 1), c = i - a * (kHeadMaxC + 1);
+    if (c < h.C) dwb_out[a * h.C + c] = (float)red[0][i];
+    else if (c == kHeadMaxC) dwb_out[NDIM * h.C + a] = (float)red[0][i];
 }
 
-static unsigned flow_grid(size_t vol)
+static int flow_grid(size_t vol, unsigned &grid)
 {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    int sms;
+    if (int rc = sm_count(sms)) return rc;
     size_t nb = (vol + 255) / 256;      // enough CTAs for every SM to hold 8; each strides over row pairs
     const size_t cap = (size_t)sms * 8;
     if (nb > cap) nb = cap;
     if (nb > kFlowMaxBlocks) nb = kFlowMaxBlocks;
-    return (unsigned)(nb < 1 ? 1 : nb);
+    grid = (unsigned)(nb < 1 ? 1 : nb);
+    return TRB_OK;
 }
 
 static int validate_flow(int ndim, int D, int H, int W)
@@ -430,9 +310,11 @@ extern "C" int trb_warp_flow(int ndim, const float *src_dev, const float *flow_d
     if (rc) return rc;
     if (!src_dev || !flow_dev || !out_dev || n_channels < 1) { set_error("null pointer / n_channels"); return TRB_ERR_ARG; }
     const size_t vol = (size_t)(ndim == 3 ? D : 1) * H * W;
+    unsigned g;
+    if ((rc = flow_grid(vol, g))) return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    if (ndim == 3) warp_flow_kernel<3><<<flow_grid(vol), 256, 0, s>>>(src_dev, flow_dev, out_dev, n_channels, D, H, W);
-    else warp_flow_kernel<2><<<flow_grid(vol), 256, 0, s>>>(src_dev, flow_dev, out_dev, n_channels, 1, H, W);
+    if (ndim == 3) warp_flow_kernel<3><<<g, 256, 0, s>>>(src_dev, flow_dev, out_dev, n_channels, D, H, W);
+    else warp_flow_kernel<2><<<g, 256, 0, s>>>(src_dev, flow_dev, out_dev, n_channels, 1, H, W);
     return check_cuda(cudaGetLastError(), "warp_flow");
 }
 
@@ -443,9 +325,11 @@ extern "C" int trb_warp_flow_vjp(int ndim, const float *src_dev, const float *fl
     if (rc) return rc;
     if (!src_dev || !flow_dev || !gout_dev || !dflow_dev) { set_error("null pointer"); return TRB_ERR_ARG; }
     const size_t vol = (size_t)(ndim == 3 ? D : 1) * H * W;
+    unsigned g;
+    if ((rc = flow_grid(vol, g))) return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    if (ndim == 3) warp_flow_vjp_kernel<3><<<flow_grid(vol), 256, 0, s>>>(src_dev, flow_dev, gout_dev, dflow_dev, D, H, W);
-    else warp_flow_vjp_kernel<2><<<flow_grid(vol), 256, 0, s>>>(src_dev, flow_dev, gout_dev, dflow_dev, 1, H, W);
+    if (ndim == 3) warp_flow_vjp_kernel<3><<<g, 256, 0, s>>>(src_dev, flow_dev, gout_dev, dflow_dev, D, H, W);
+    else warp_flow_vjp_kernel<2><<<g, 256, 0, s>>>(src_dev, flow_dev, gout_dev, dflow_dev, 1, H, W);
     return check_cuda(cudaGetLastError(), "warp_flow_vjp");
 }
 
@@ -463,7 +347,8 @@ extern "C" int trb_flow_loss_grad(int ndim, const float *moving_dev, const float
     const size_t vol = (size_t)(ndim == 3 ? D : 1) * H * W;
     cudaStream_t s = (cudaStream_t)stream;
     double *ws = (double *)workspace_dev;
-    const unsigned g = flow_grid(vol);
+    unsigned g;
+    if ((rc = flow_grid(vol, g))) return rc;
     if (w_ncc == 0.f) {                 // no global moments needed: one fused pass (32 B/voxel instead of 52)
         if (ndim == 3) flow_mse_fused_kernel<3><<<g, 256, 0, s>>>(moving_dev, target_dev, flow_dev, dflow_dev, warped_dev_or_null, D, H, W, w_mse, ws, loss_dev);
         else flow_mse_fused_kernel<2><<<g, 256, 0, s>>>(moving_dev, target_dev, flow_dev, dflow_dev, warped_dev_or_null, 1, H, W, w_mse, ws, loss_dev);
@@ -497,7 +382,8 @@ extern "C" int trb_flow_head_forward(int ndim, const float *moving_dev, const fl
     h.lz = ndim == 3 ? lo(D, fd) : 0; h.ly = lo(H, fh); h.lx = lo(W, fw);
     h.Wd = w_dev; h.bd = b_dev;
     const size_t vol = (size_t)(ndim == 3 ? D : 1) * H * W;
-    const unsigned g = flow_grid(vol);
+    unsigned g;
+    if ((rc = flow_grid(vol, g))) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     if (ndim == 3) flow_head_forward_kernel<3><<<g, 256, 0, s>>>(moving_dev, target_dev, h, flow_out_dev, D, H, W, w_mse, w_ncc, (double *)workspace_dev, loss_dev);
     else flow_head_forward_kernel<2><<<g, 256, 0, s>>>(moving_dev, target_dev, h, flow_out_dev, 1, H, W, w_mse, w_ncc, (double *)workspace_dev, loss_dev);
@@ -519,7 +405,8 @@ extern "C" int trb_flow_head_backward(int ndim, const float *moving_dev, const f
     h.lz = ndim == 3 ? lo(D, fd) : 0; h.ly = lo(H, fh); h.lx = lo(W, fw);
     h.Wd = w_dev; h.bd = nullptr;
     const size_t vol = (size_t)(ndim == 3 ? D : 1) * H * W;
-    const unsigned g = flow_grid(vol);
+    unsigned g;
+    if ((rc = flow_grid(vol, g))) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     if (ndim == 3) flow_head_backward_kernel<3><<<g, 256, 0, s>>>(moving_dev, target_dev, flow_dev, h, dfeat_dev, D, H, W, (double *)workspace_dev, dwb_dev);
     else flow_head_backward_kernel<2><<<g, 256, 0, s>>>(moving_dev, target_dev, flow_dev, h, dfeat_dev, 1, H, W, (double *)workspace_dev, dwb_dev);

@@ -27,26 +27,13 @@ static int in_chunks(long long S)
     return (int)c;
 }
 
-__device__ __forceinline__ void block_sum2(double &a, double &b, double (*sh)[2])
-{
-    a = warp_sum(a); b = warp_sum(b);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (lane == 0) { sh[warp][0] = a; sh[warp][1] = b; }
-    __syncthreads();
-    a = 0.0; b = 0.0;
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int w = 0; w < 8; ++w) { a += sh[w][0]; b += sh[w][1]; }
-    }
-}
-
 // grid (chunks, instances).  BWD = false: (sum v, sum v^2) of v = relu?(x);  BWD = true: (sum dy, sum dy*y), y from x and stats.
 template <bool BWD, bool VEC>
 __global__ void __launch_bounds__(256) instnorm_sums_kernel(const float *__restrict__ x, const float *__restrict__ gate,
                                                              const float *__restrict__ dy, long long S,
                                                              int relu, const float *__restrict__ stats, double *__restrict__ part)
 {
-    __shared__ double sh[8][2];
+    __shared__ double sh[kWarps][2];
     const int chunk = blockIdx.x, chunks = gridDim.x, inst = blockIdx.y;
     const long long i0 = S * chunk / chunks, i1 = S * (chunk + 1) / chunks;
     const float *xi = x + (size_t)inst * S;
@@ -80,24 +67,22 @@ __global__ void __launch_bounds__(256) instnorm_sums_kernel(const float *__restr
             if (++n == 32) { A += (double)a; B += (double)b; a = b = 0.f; n = 0; }
         }
     }
-    A += (double)a; B += (double)b;
-    block_sum2(A, B, sh);
-    if (threadIdx.x == 0) {
-        double *o = part + ((size_t)inst * chunks + chunk) * 2;
-        o[0] = A; o[1] = B;
-    }
+    const double AB[2] = {A + (double)a, B + (double)b};
+    const double t = block_sum(AB, sh);
+    if (threadIdx.x < 2) __stcg(part + ((size_t)inst * chunks + chunk) * 2 + threadIdx.x, t);
 }
 
 // grid (instances).  FWD: stats[inst] = (mean, rstd).  BWD: coef[inst] = (mean dy, mean dy*y).
 __global__ void __launch_bounds__(256) instnorm_finalise_kernel(const double *__restrict__ part, int chunks, long long S, float eps, int bwd,
                                                                  float *__restrict__ out)
 {
-    __shared__ double sh[8][2];
+    __shared__ double sh[kWarps][2];
     const int inst = blockIdx.x;
     const double *p = part + (size_t)inst * chunks * 2;
-    double A = 0.0, B = 0.0;
-    for (int c = threadIdx.x; c < chunks; c += 256) { A += p[2 * c]; B += p[2 * c + 1]; }
-    block_sum2(A, B, sh);
+    double AB[2] = {0.0, 0.0};
+    for (int c = threadIdx.x; c < chunks; c += 256) { AB[0] += p[2 * c]; AB[1] += p[2 * c + 1]; }
+    block_sum_all(AB, sh);
+    const double A = AB[0], B = AB[1];
     if (threadIdx.x == 0) {
         const double n = (double)S;
         if (bwd) { out[2 * inst] = (float)(A / n); out[2 * inst + 1] = (float)(B / n); }

@@ -259,8 +259,7 @@ __global__ void __launch_bounds__(256) nmi_epilogue_kernel(const double *__restr
                                                             float *__restrict__ gtab, double *__restrict__ scal,
                                                             double *__restrict__ loss_out)
 {
-    __shared__ double sh[8];
-    __shared__ bool is_last;
+    __shared__ double sh[kWarps][1];
     const int b = threadIdx.x, k = blockIdx.x;
     const size_t hs = (size_t)K * kBins;
     const double eps = 1e-10, ln2 = 0.6931471805599453;
@@ -283,13 +282,13 @@ __global__ void __launch_bounds__(256) nmi_epilogue_kernel(const double *__restr
     const double H1 = momT ? expand_moments(r1, yT) : r1[b];
     const double H2 = momWJ ? expand_moments(r2, yW) : r2[b];
     const double HJ = momWJ ? expand_moments(r3, yJ) + expand_moments(r4, yJ) : r3[b] + r4[b];
-    const double S1 = block_sum256(H1, sh), S2 = block_sum256(H2, sh), SJ = block_sum256(HJ, sh);
+    const double S1 = block_sum_all(H1, sh), S2 = block_sum_all(H2, sh), SJ = block_sum_all(HJ, sh);
     const double p1 = H1 / S1, p2 = H2 / S2, pj = HJ / SJ;
     const double l2 = log2(p2 + eps), lj = log2(pj + eps);
-    const double E1 = block_sum256(p1 * log2(p1 + eps), sh);
-    const double E2 = block_sum256(p2 * l2, sh), EJ = block_sum256(pj * lj, sh);
+    const double E1 = block_sum_all(p1 * log2(p1 + eps), sh);
+    const double E2 = block_sum_all(p2 * l2, sh), EJ = block_sum_all(pj * lj, sh);
     const double d2 = l2 + p2 / ((p2 + eps) * ln2), dj = lj + pj / ((pj + eps) * ln2);      // dE/dp_b
-    const double A2 = block_sum256(p2 * d2, sh), AJ = block_sum256(pj * dj, sh);
+    const double A2 = block_sum_all(p2 * d2, sh), AJ = block_sum_all(pj * dj, sh);
     const double den = E1 + E2, mi = den - EJ;
     const double nmi = 2.0 * mi / den;
     const double dev = nmi - 1.0;
@@ -302,7 +301,7 @@ __global__ void __launch_bounds__(256) nmi_epilogue_kernel(const double *__restr
         // Gamma_m = sum_b G_b y_b^m / m!, stored as -Gamma_m/h in gW[m] / gJ[m]; the range centres in cW[0] / cJ[0]
         double tw = G2, tj = GJ;
         for (int m = 0; m < kMom; ++m) {
-            const double gw = block_sum256(tw, sh), gj = block_sum256(tj, sh);
+            const double gw = block_sum_all(tw, sh), gj = block_sum_all(tj, sh);
             if (b == 0) { tab[kBins + m] = (float)(-gw / (double)h); tab[4 * kBins + m] = (float)(-gj / (double)h); }
             tw *= yW / (double)(m + 1); tj *= yJ / (double)(m + 1);
         }
@@ -316,14 +315,8 @@ __global__ void __launch_bounds__(256) nmi_epilogue_kernel(const double *__restr
     }
     // chunk term -> scal[k]; the last block adds them in chunk order
     unsigned *ticket = reinterpret_cast<unsigned *>(scal + 8);
-    if (b == 0) {
-        __stcg(scal + k, fabs(dev));
-        __threadfence();
-        is_last = atomicAdd(ticket, 1u) == (unsigned)K - 1;
-    }
-    __syncthreads();
-    if (is_last && b == 0) {
-        __threadfence();
+    if (b == 0) __stcg(scal + k, fabs(dev));
+    if (last_to_arrive(ticket, K) && b == 0) {
         double loss = 0.0;
         for (int c = 0; c < K; ++c) loss += __ldcg(scal + c);
         *loss_out = weight * alpha * loss / (double)K;

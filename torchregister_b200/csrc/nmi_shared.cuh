@@ -94,18 +94,6 @@ __device__ __forceinline__ void hermite_chain(float s, float mid, float inv_h, F
     }
 }
 
-__device__ __forceinline__ double block_sum256(double v, double *sh)
-{
-    v = warp_sum(v);
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = v;
-    __syncthreads();
-    double r = 0.0;
-#pragma unroll
-    for (int w = 0; w < 8; ++w) r += sh[w];
-    return r;
-}
-
 // a histogram kept in moment form (M_0..M_11) evaluated at the bin with reduced centre y = (c_b - mid)/h, in fp64
 __device__ __forceinline__ double expand_moments(const double *__restrict__ row, double y)
 {

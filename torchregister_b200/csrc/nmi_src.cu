@@ -145,7 +145,7 @@ __global__ void __launch_bounds__(256) nmi_src_moments_kernel(const float *__res
                                                                float mid, float inv_h, double *__restrict__ part,
                                                                int *__restrict__ keys, int key_off)
 {
-    __shared__ double red[8][kPow];
+    __shared__ double red[kWarps][kPow];
     __shared__ float rmn[8], rmx[8];
     __shared__ int mzk[kMaxChunkSlices];
     const int b = blockIdx.x, B = gridDim.x, k = blockIdx.y, K = gridDim.y, cs = kRes / K, pair = blockIdx.z;
@@ -196,25 +196,13 @@ __global__ void __launch_bounds__(256) nmi_src_moments_kernel(const float *__res
             }
     }
 #pragma unroll
-    for (int m = 0; m < kPow; ++m) {
-        const double sm = warp_sum((double)a[m]);
-        if (lane == 0) red[warp][m] = sm;
-    }
-#pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         mn = fminf(mn, __shfl_xor_sync(kFull, mn, o));
         mx = fmaxf(mx, __shfl_xor_sync(kFull, mx, o));
     }
     if (lane == 0) { rmn[warp] = mn; rmx[warp] = mx; }
-    __syncthreads();
-    if (threadIdx.x < kMomPad) {
-        double sm = 0.0;
-        if (threadIdx.x < kPow) {
-#pragma unroll
-            for (int w = 0; w < 8; ++w) sm += red[w][threadIdx.x];
-        }
-        part[(((size_t)pair * K + k) * B + b) * kMomPad + threadIdx.x] = sm;
-    }
+    const double sm = block_sum(a, red);                        // its barrier also publishes rmn / rmx
+    if (threadIdx.x < kMomPad) part[(((size_t)pair * K + k) * B + b) * kMomPad + threadIdx.x] = sm;
     if (threadIdx.x == 32) {
 #pragma unroll
         for (int w = 0; w < 8; ++w) { mn = fminf(mn, rmn[w]); mx = fmaxf(mx, rmx[w]); }
@@ -222,26 +210,6 @@ __global__ void __launch_bounds__(256) nmi_src_moments_kernel(const float *__res
             atomicMin(keys + 4 * pair + key_off, float_key(mn));
             atomicMax(keys + 4 * pair + key_off + 1, float_key(mx));
         }
-    }
-}
-
-template <int N>
-__device__ __forceinline__ void block_sum256_n(double (&v)[N], double (*sh)[8])
-{
-#pragma unroll
-    for (int i = 0; i < N; ++i) v[i] = warp_sum(v[i]);
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) {
-#pragma unroll
-        for (int i = 0; i < N; ++i) sh[i][threadIdx.x >> 5] = v[i];
-    }
-    __syncthreads();
-#pragma unroll
-    for (int i = 0; i < N; ++i) {
-        double r = 0.0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) r += sh[i][w];
-        v[i] = r;
     }
 }
 
@@ -260,8 +228,7 @@ __global__ void __launch_bounds__(256) nmi_src_epilogue_kernel(const double *__r
 {
     __shared__ double fold[16][kMomPad + 1];
     __shared__ double rowW[kMomPad];
-    __shared__ double sh[kPow + 1][8];
-    __shared__ bool is_last;
+    __shared__ double sh[kWarps][kPow + 1];
     const int b = threadIdx.x, k = blockIdx.x, pair = blockIdx.y, K = gridDim.x;
     {
         const int col = b & 15, ln = b >> 4;
@@ -309,13 +276,13 @@ __global__ void __launch_bounds__(256) nmi_src_epilogue_kernel(const double *__r
         }
     }
     const double H1 = hs[0], H2 = hs[1], HJ = hs[2];
-    block_sum256_n<3>(hs, sh);
+    block_sum_all(hs, sh);
     const double S1 = hs[0], S2 = hs[1], SJ = hs[2];
     const double p1 = H1 / S1, p2 = H2 / S2, pj = HJ / SJ;
     const double l2 = log2(p2 + eps), lj = log2(pj + eps);
     const double d2 = l2 + p2 / ((p2 + eps) * ln2), dj = lj + pj / ((pj + eps) * ln2);      // dE/dp_b
     double es[5] = {p1 * log2(p1 + eps), p2 * l2, pj * lj, p2 * d2, pj * dj};
-    block_sum256_n<5>(es, sh);
+    block_sum_all(es, sh);
     const double E1 = es[0], E2 = es[1], EJ = es[2], A2 = es[3], AJ = es[4];
     const double den = E1 + E2, mi = den - EJ;
     const double nmi = 2.0 * mi / den;
@@ -327,7 +294,7 @@ __global__ void __launch_bounds__(256) nmi_src_epilogue_kernel(const double *__r
     double lm[kPow + 1];
 #pragma unroll
     for (int m = 0; m <= kPow; ++m) lm[m] = G2 * pW[m] + GJ * pJ[m];
-    block_sum256_n<kPow + 1>(lm, sh);
+    block_sum_all(lm, sh);
     if (b == 0) {
         float *tab = gtab + ((size_t)pair * K + k) * kMomPad;
 #pragma unroll
@@ -335,14 +302,8 @@ __global__ void __launch_bounds__(256) nmi_src_epilogue_kernel(const double *__r
     }
     // chunk term -> scal[k]; the last block of the pair adds them in chunk order
     unsigned *ticket = reinterpret_cast<unsigned *>(scal + 8);
-    if (b == 0) {
-        __stcg(scal + k, fabs(dev));
-        __threadfence();
-        is_last = atomicAdd(ticket, 1u) == (unsigned)K - 1;
-    }
-    __syncthreads();
-    if (is_last && b == 0) {
-        __threadfence();
+    if (b == 0) __stcg(scal + k, fabs(dev));
+    if (last_to_arrive(ticket, K) && b == 0) {
         double loss = 0.0;
         for (int c = 0; c < K; ++c) loss += __ldcg(scal + c);
         loss = weight * alpha * loss / (double)K;

@@ -134,7 +134,7 @@ __global__ void __launch_bounds__(256) thinconv_wgrad_kernel(const float *__rest
                                                               int co_groups, double *__restrict__ part)
 {
     constexpr int NA = 9 * COG + COG, XB = 4;
-    __shared__ double sh[8][NA];
+    __shared__ double sh[kWarps][NA];
     const int OD = D - 2, OH = H - 2, OW = W - 2;
     const int g = blockIdx.y, cg = g % co_groups, cd = g / co_groups, ci = cd / 3, dz = cd - ci * 3;
     const size_t HW = (size_t)H * W, vol = HW * D, OHW = (size_t)OH * OW, ovol = OHW * OD;
@@ -179,17 +179,9 @@ __global__ void __launch_bounds__(256) thinconv_wgrad_kernel(const float *__rest
         }
     }
 #pragma unroll
-    for (int i = 0; i < NA; ++i) {
-        const double v = warp_sum(A[i] + (double)a[i]);
-        if (lane == 0) sh[warp][i] = v;
-    }
-    __syncthreads();
-    if (threadIdx.x < NA) {
-        double v = 0.0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) v += sh[w][threadIdx.x];
-        part[((size_t)g * gridDim.x + blockIdx.x) * NA + threadIdx.x] = v;
-    }
+    for (int i = 0; i < NA; ++i) A[i] += (double)a[i];
+    const double v = block_sum(A, sh);
+    if (threadIdx.x < NA) part[((size_t)g * gridDim.x + blockIdx.x) * NA + threadIdx.x] = v;
 }
 
 // dw[co][ci][dz][dy][dx] and db[co] from the block partials, fixed order
@@ -394,7 +386,7 @@ __global__ void __launch_bounds__(256) pointconv_wgrad_kernel(const float *__res
                                                                int OD, int OH, int OW, int stride, double *__restrict__ part)
 {
     constexpr int NA = CI * CO + CO;
-    __shared__ double sh[8][NA];
+    __shared__ double sh[kWarps][NA];
     const size_t vol = (size_t)D * H * W, ovol = (size_t)OD * OH * OW;
     float a[NA];
     double A[NA];
@@ -426,31 +418,20 @@ __global__ void __launch_bounds__(256) pointconv_wgrad_kernel(const float *__res
             since = 0;
         }
     }
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
-    for (int k = 0; k < NA; ++k) {
-        const double s = warp_sum(A[k] + (double)a[k]);
-        if (lane == 0) sh[warp][k] = s;
-    }
-    __syncthreads();
-    if (threadIdx.x < NA) {
-        double s = 0.0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) s += sh[w][threadIdx.x];
-        part[(size_t)blockIdx.x * NA + threadIdx.x] = s;
-    }
+    for (int k = 0; k < NA; ++k) A[k] += (double)a[k];
+    const double s = block_sum(A, sh);
+    if (threadIdx.x < NA) part[(size_t)blockIdx.x * NA + threadIdx.x] = s;
 }
 
 // one warp per sum: lanes stride over the block partials (fixed order), then a shuffle tree
 __global__ void pointconv_wgrad_final_kernel(const double *__restrict__ part, int blocks, int CI, int CO, float *__restrict__ gw,
                                              float *__restrict__ gb)
 {
-    const int NA = CI * CO + CO, k = blockIdx.x, lane = threadIdx.x;
+    const int NA = CI * CO + CO, k = blockIdx.x;
     if (k >= NA) return;
-    double s = 0.0;
-    for (int b = lane; b < blocks; b += 32) s += part[(size_t)b * NA + k];
-    s = warp_sum(s);
-    if (lane == 0) {
+    const double s = fold_blocks(part, blocks, NA, k);
+    if (threadIdx.x == 0) {
         if (k < CI * CO) gw[k] = (float)s;
         else if (gb) gb[k - CI * CO] = (float)s;
     }
@@ -595,7 +576,7 @@ __global__ void __launch_bounds__(256) upconv2_wgrad_kernel(const float *__restr
                                                              double *__restrict__ part)
 {
     constexpr int NA = 8 * CO + CO;
-    __shared__ double sh[8][NA];
+    __shared__ double sh[kWarps][NA];
     const int ci = blockIdx.y;
     const size_t vol = (size_t)D * H * W, ovol = vol * 8;
     const int OW = 2 * W, OH = 2 * H;
@@ -626,32 +607,21 @@ __global__ void __launch_bounds__(256) upconv2_wgrad_kernel(const float *__restr
             since = 0;
         }
     }
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
-    for (int k = 0; k < NA; ++k) {
-        const double s = warp_sum(A[k] + (double)acc[k]);
-        if (lane == 0) sh[warp][k] = s;
-    }
-    __syncthreads();
-    if (threadIdx.x < NA) {
-        double s = 0.0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) s += sh[w][threadIdx.x];
-        part[((size_t)ci * gridDim.x + blockIdx.x) * NA + threadIdx.x] = s;
-    }
+    for (int k = 0; k < NA; ++k) A[k] += (double)acc[k];
+    const double s = block_sum(A, sh);
+    if (threadIdx.x < NA) part[((size_t)ci * gridDim.x + blockIdx.x) * NA + threadIdx.x] = s;
 }
 
 // one warp per entry: gw[ci][co][8] (k < 8*CO of group ci) and gb[co] (from group 0)
 __global__ void upconv2_wgrad_final_kernel(const double *__restrict__ part, int blocks, int CI, int CO, float *__restrict__ gw, float *__restrict__ gb)
 {
-    const int NA = 8 * CO + CO, e = blockIdx.x, lane = threadIdx.x;
+    const int NA = 8 * CO + CO, e = blockIdx.x;
     int ci, k;
     if (e < CI * CO * 8) { ci = e / (CO * 8); k = e - ci * CO * 8; }
     else { ci = 0; k = 8 * CO + (e - CI * CO * 8); }
-    double s = 0.0;
-    for (int b = lane; b < blocks; b += 32) s += part[((size_t)ci * blocks + b) * NA + k];
-    s = warp_sum(s);
-    if (lane == 0) {
+    const double s = fold_blocks(part + (size_t)ci * blocks * NA, blocks, NA, k);
+    if (threadIdx.x == 0) {
         if (e < CI * CO * 8) gw[e] = (float)s;          // [ci][co][a][b][c] is exactly e
         else if (gb) gb[e - CI * CO * 8] = (float)s;
     }

@@ -231,9 +231,8 @@ int launch_warp_affine_tma(const float *moving, float *out, int n_pairs, int n_c
     wp.t.tiles_x = (W + TX - 1) / TX; wp.t.tiles_y = (H + TY - 1) / TY; wp.t.tiles_z = (D + TZ - 1) / TZ;
     wp.t.cols_per_pair = wp.t.tiles_x * wp.t.tiles_y;
     wp.theta = theta_dev; wp.out = out; wp.n_channels = n_channels;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    int sms;
+    if ((rc = sm_count(sms))) return rc;
     const long long total_cols = (long long)n_items * wp.t.cols_per_pair;
     long long grid_ll = sms;
     if (grid_ll > total_cols * wp.t.tiles_z) grid_ll = total_cols * wp.t.tiles_z;
