@@ -45,6 +45,7 @@ extern "C" {
 #define TRB_FLAG_LARGE_ROTATION 1   /* trb_affine_optim_ex / trb_warp_affine_batch: see there */
 #define TRB_FLAG_PAIR_VOLUME 2      /* with TRB_FLAG_LARGE_ROTATION: a pair volume is attached to the workspace (trb_affine_attach_pairs) */
 #define TRB_FLAG_QUAD_VOLUME 4      /* with TRB_FLAG_LARGE_ROTATION: a quad volume is attached instead (trb_affine_build_quads) */
+#define TRB_FLAG_NEAREST 8          /* trb_warp_affine_batch / trb_warp_flow_ex: nearest-neighbour sampling (label maps) */
 
 /* Per-pair optimiser state: TRB_STATE_FLOATS fp32 values, device resident.
  *   [ 0..11] params        (rigid: 6|3 used, affine: 12|6 used)
@@ -209,7 +210,9 @@ int trb_warp_affine(int ndim, const float *moving_dev, float *out_dev, int n_cha
 
 /* The same for a batch: n_pairs pairs of n_channels volumes each ([n_pairs][n_channels][D][H][W] contiguous), theta_dev
  * [n_pairs][12|6], ONE launch.  3-D shapes with W % 4 == 0, W >= 32, H >= 16 take the TMA-staged kernel (csrc/warp_tma.cu);
- * flags: TRB_FLAG_LARGE_ROTATION = theta is known to rotate by more than a few degrees (gather kernel instead). */
+ * flags: TRB_FLAG_LARGE_ROTATION = theta is known to rotate by more than a few degrees (gather kernel instead);
+ * TRB_FLAG_NEAREST = grid_sample(mode='nearest'): the source coordinate rounded half to even, zero outside the volume,
+ * so only input values and 0 appear in out (label maps).  Same path selection with or without it. */
 int trb_warp_affine_batch(int ndim, const float *moving_dev, float *out_dev, int n_pairs, int n_channels,
                           int D, int H, int W, const float *theta_dev,
                           const float *xb_dev, const float *yb_dev, const float *zb_dev, int flags, void *stream);
@@ -237,6 +240,22 @@ size_t trb_flow_workspace_bytes(void);
  * flow_register.deform (warpings.py:238-242) and Register.__call__ (torchregister.py:124-125). */
 int trb_warp_flow(int ndim, const float *src_dev, const float *flow_dev, float *out_dev, int n_channels,
                   int D, int H, int W, void *stream);
+
+/* The same with option flags: TRB_FLAG_NEAREST = grid_sample(mode='nearest', align_corners=True) on the reference's
+ * grid, bit for bit (label maps); 0 = trb_warp_flow. */
+int trb_warp_flow_ex(int ndim, const float *src_dev, const float *flow_dev, float *out_dev, int n_channels,
+                     int D, int H, int W, int flags, void *stream);
+
+/* Jacobian determinant of phi(p) = p + u(p), u = flow_dev in voxel units (the layout above).  J_ij = delta_ij + du_i/dp_j
+ * with numpy.gradient's differences (central inside, one-sided at both ends; every spatial axis >= 2, else TRB_ERR_ARG),
+ * formed in fp64 with the 3x3 (2x2) determinant.  det_out_dev (nullable): the field as fp32 [D][H][W].
+ * stats_out_dev (dev, TRB_JAC_NSTATS doubles): n det <= 0, n non-finite det, min det, max det, sum det, sum det^2,
+ * sum L, sum L^2 with L = log(clamp(det, 1e-9, 1e9)); all but the non-finite count are over finite det only.  Sums in a
+ * fixed order: the same bits on every run.  workspace: trb_flow_workspace_bytes() (its ticket must be zero, as for the
+ * flow calls; the call leaves it so). */
+#define TRB_JAC_NSTATS 8
+int trb_flow_jacobian(int ndim, const float *flow_dev, int D, int H, int W, float *det_out_dev, double *stats_out_dev,
+                      void *workspace_dev, size_t workspace_bytes, void *stream);
 
 /* dflow = J^T gout for the warp above (autograd of utils.py:365 w.r.t. flow);
  * used when the caller supplies its own criterion (torchregister.py:71-73). */

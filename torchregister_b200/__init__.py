@@ -9,6 +9,7 @@ hot path of AgamChopra/TorchRegister, behind the reference's own API:
 from .utils import *            # noqa: F401,F403   (mirrors TR/__init__.py:1-3 star exports)
 from .warpings import *         # noqa: F401,F403
 from .torchregister import Register   # noqa: F401
-from . import functional, synth      # noqa: F401
+from .metrics import jacobian_determinant, dice   # noqa: F401
+from . import functional, synth, metrics      # noqa: F401
 
 __version__ = '0.1.0'

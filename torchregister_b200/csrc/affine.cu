@@ -198,12 +198,13 @@ __global__ void affine_init_state_kernel(float *state, int n_pairs, int mode)
 }
 
 // ---- forward-only warp (get_affine_warp, warpings.py:18-26) ------------------------------
-template <int NDIM>
-__global__ void __launch_bounds__(256) warp_affine_kernel(const float *__restrict__ moving, float *__restrict__ out,
-                                                           int n_channels, int D, int H, int W,
-                                                           const float *__restrict__ theta,
-                                                           const float *__restrict__ xb, const float *__restrict__ yb,
-                                                           const float *__restrict__ zb)
+// NEAREST: grid_sample(mode='nearest'): the source coordinate rounded half to even, one predicated load per channel
+template <int NDIM, bool NEAREST>
+__device__ __forceinline__ void warp_affine_body(const float *__restrict__ moving, float *__restrict__ out,
+                                                 int n_channels, int D, int H, int W,
+                                                 const float *__restrict__ theta,
+                                                 const float *__restrict__ xb, const float *__restrict__ yb,
+                                                 const float *__restrict__ zb)
 {
     constexpr int NC = NDIM + 1, NT = NDIM * NC;
     const size_t HW = (size_t)H * W, vol = HW * (NDIM == 3 ? D : 1);
@@ -222,6 +223,12 @@ __global__ void __launch_bounds__(256) warp_affine_kernel(const float *__restric
             const float ix = fmaf(th[0] * hw, xv, fmaf(th[1] * yv + th[2] * zv + th[3] + 1.f, hw, -0.5f));
             const float iy = fmaf(th[4] * hh, xv, fmaf(th[5] * yv + th[6] * zv + th[7] + 1.f, hh, -0.5f));
             const float iz = fmaf(th[8] * hd, xv, fmaf(th[9] * yv + th[10] * zv + th[11] + 1.f, hd, -0.5f));
+            if constexpr (NEAREST) {
+                long long o;
+                const bool v = nearest_offset(D, H, W, ix, iy, iz, o);
+                for (int c = 0; c < n_channels; ++c) out[(size_t)c * vol + idx] = v ? __ldg(moving + (size_t)c * vol + o) : 0.f;
+                return;
+            }
             const float fx = floorf(ix), fy = floorf(iy), fz = floorf(iz);
             Cell3 k;
             k.tx = ix - fx; k.ty = iy - fy; k.tz = iz - fz;
@@ -247,6 +254,12 @@ __global__ void __launch_bounds__(256) warp_affine_kernel(const float *__restric
         } else {
             const float ix = fmaf(th[0] * hw, xv, fmaf(th[1] * yv + th[2] + 1.f, hw, -0.5f));
             const float iy = fmaf(th[3] * hh, xv, fmaf(th[4] * yv + th[5] + 1.f, hh, -0.5f));
+            if constexpr (NEAREST) {
+                long long o;
+                const bool v = nearest_offset(1, H, W, ix, iy, 0.f, o);
+                for (int c = 0; c < n_channels; ++c) out[(size_t)c * vol + idx] = v ? __ldg(moving + (size_t)c * vol + o) : 0.f;
+                return;
+            }
             const float fx = floorf(ix), fy = floorf(iy);
             Cell2 k;
             k.tx = ix - fx; k.ty = iy - fy;
@@ -265,6 +278,24 @@ __global__ void __launch_bounds__(256) warp_affine_kernel(const float *__restric
             }
         }
     });
+}
+template <int NDIM>
+__global__ void __launch_bounds__(256) warp_affine_kernel(const float *__restrict__ moving, float *__restrict__ out,
+                                                           int n_channels, int D, int H, int W,
+                                                           const float *__restrict__ theta,
+                                                           const float *__restrict__ xb, const float *__restrict__ yb,
+                                                           const float *__restrict__ zb)
+{
+    warp_affine_body<NDIM, false>(moving, out, n_channels, D, H, W, theta, xb, yb, zb);
+}
+template <int NDIM>
+__global__ void __launch_bounds__(256) warp_affine_nearest_kernel(const float *__restrict__ moving, float *__restrict__ out,
+                                                                   int n_channels, int D, int H, int W,
+                                                                   const float *__restrict__ theta,
+                                                                   const float *__restrict__ xb, const float *__restrict__ yb,
+                                                                   const float *__restrict__ zb)
+{
+    warp_affine_body<NDIM, true>(moving, out, n_channels, D, H, W, theta, xb, yb, zb);
 }
 
 __global__ void vjp_extract_kernel(const double *moments, double *dtheta, int ndim, int D, int H, int W)
@@ -675,16 +706,23 @@ extern "C" int trb_warp_affine_batch(int ndim, const float *moving_dev, float *o
     cudaStream_t s = (cudaStream_t)stream;
     // 3-D: TMA-staged tiles unless the caller knows theta is a large rotation (then the gathers of the one-thread-per-
     // voxel kernel, which keeps the whole L1, are the better path)
+    const bool nearest = flags & TRB_FLAG_NEAREST;
     if (ndim == 3 && !g_force_direct && !(flags & TRB_FLAG_LARGE_ROTATION) &&
         warp_tma_eligible(moving_dev, out_dev, n_pairs * n_channels, (long long)vol, D, H, W))
-        return launch_warp_affine_tma(moving_dev, out_dev, n_pairs, n_channels, D, H, W, theta_dev, xb_dev, yb_dev, s);
+        return launch_warp_affine_tma(moving_dev, out_dev, n_pairs, n_channels, D, H, W, theta_dev, xb_dev, yb_dev, nearest, s);
     int sms;
     if ((rc = sm_count(sms))) return rc;
     size_t nb = (vol + 255) / 256;
     if (nb > (size_t)sms * 16) nb = (size_t)sms * 16;
     const dim3 grid((unsigned)nb, (unsigned)n_pairs);
-    if (ndim == 3) warp_affine_kernel<3><<<grid, 256, 0, s>>>(moving_dev, out_dev, n_channels, D, H, W, theta_dev, xb_dev, yb_dev, zb_dev);
-    else warp_affine_kernel<2><<<grid, 256, 0, s>>>(moving_dev, out_dev, n_channels, 1, H, W, theta_dev, xb_dev, yb_dev, zb_dev);
+    if (nearest) {
+        if (ndim == 3) warp_affine_nearest_kernel<3><<<grid, 256, 0, s>>>(moving_dev, out_dev, n_channels, D, H, W, theta_dev, xb_dev, yb_dev, zb_dev);
+        else warp_affine_nearest_kernel<2><<<grid, 256, 0, s>>>(moving_dev, out_dev, n_channels, 1, H, W, theta_dev, xb_dev, yb_dev, zb_dev);
+    } else if (ndim == 3) {
+        warp_affine_kernel<3><<<grid, 256, 0, s>>>(moving_dev, out_dev, n_channels, D, H, W, theta_dev, xb_dev, yb_dev, zb_dev);
+    } else {
+        warp_affine_kernel<2><<<grid, 256, 0, s>>>(moving_dev, out_dev, n_channels, 1, H, W, theta_dev, xb_dev, yb_dev, zb_dev);
+    }
     return check_cuda(cudaGetLastError(), "warp_affine");
 }
 

@@ -30,7 +30,7 @@ const char *persist_status();
 // TMA-staged forward warp (warp_tma.cu)
 bool warp_tma_eligible(const float *moving, const float *out, int n_items, long long vol, int D, int H, int W);
 int launch_warp_affine_tma(const float *moving, float *out, int n_pairs, int n_channels, int D, int H, int W,
-                           const float *theta_dev, const float *xb, const float *yb, cudaStream_t stream);
+                           const float *theta_dev, const float *xb, const float *yb, bool nearest, cudaStream_t stream);
 
 struct AffineParams {
     const float *moving, *target;

@@ -165,6 +165,17 @@ __device__ __forceinline__ BoxCells box_cells(float Mrel, float2 ix, float2 iy, 
                       __ffma2_rn(f2(kIdxScale * (float)BX), fy, __ffma2_rn(f2(kIdxScale), fx, f2(Mrel))));
     return b;
 }
+// The nearest-neighbour twin (grid_sample mode='nearest'): box indices of the voxels at ix, iy, iz rounded half to even,
+// the same add in round-to-nearest mode.  The rounded index lies in {floor, floor + 1}, so a box that holds the cells
+// holds these voxels too.
+template <int BX, int BY>
+__device__ __forceinline__ float2 box_nearest(float Mrel, float2 ix, float2 iy, float2 iz)
+{
+    const float2 M = f2(kMagic), nM = f2(-kMagic);
+    const float2 rx = __fadd2_rn(__fadd2_rn(ix, M), nM), ry = __fadd2_rn(__fadd2_rn(iy, M), nM), rz = __fadd2_rn(__fadd2_rn(iz, M), nM);
+    return __ffma2_rn(f2(kIdxScale * (float)(BX * BY)), rz,
+                      __ffma2_rn(f2(kIdxScale * (float)BX), ry, __ffma2_rn(f2(kIdxScale), rx, f2(Mrel))));
+}
 // smem byte address of a cell's corner; box_m: smem byte address of the staged box.  The box-relative linear index
 // is formed in fp32 and scaled by 2^-22 onto [2, 4): exact, and the bit pattern is 0x40000000 + index, so (bits << 2)
 // IS the byte offset (the 0x4 wraps away)

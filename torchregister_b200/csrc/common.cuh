@@ -180,6 +180,17 @@ __device__ __forceinline__ float flow_pos(const AxisMap &m, int i, float f)
     return __fmul_rn(__fmul_rn(__fadd_rn(nrm, 1.f), 0.5f), m.d);
 }
 
+// The same round trip as torch evaluates it on a CUDA device: there a division by a Python scalar is a multiply by the
+// scalar's fp32 reciprocal (PyTorch's div_true_kernel_cuda), which differs from the IEEE quotient in the last bit for some
+// positions.  A bilinear sample moves by ~1e-7 of a voxel with that bit; a nearest sample can flip at an exact half-voxel
+// position, so the nearest flow warp follows the device's grid.
+__device__ __forceinline__ float flow_pos_rcp(const AxisMap &m, int i, float f)
+{
+    const float loc = (float)i + f;
+    const float nrm = 2.f * (__fmul_rn(loc, m.r) - 0.5f);
+    return __fmul_rn(__fmul_rn(__fadd_rn(nrm, 1.f), 0.5f), m.d);
+}
+
 // floor and fraction without the quarter-rate conversion pipe: adding 1.5*2^23 rounding down leaves floor(p) in the
 // low mantissa bits (exact for |p| < 2^22; anything further out — inf and NaN included — lands on an index no volume
 // reaches, i.e. on the zero padding).
@@ -194,6 +205,24 @@ __device__ __forceinline__ void floor_frac(float p, int &i0, float &t)
 {
     float fl;
     floor_frac(p, i0, t, fl);
+}
+
+// grid_sample(mode='nearest')'s source index: p rounded half to even, as torch's nearbyint does.  The same 1.5*2^23 add
+// as floor_frac, in round-to-nearest mode, rather than __float2int_rn: the conversion maps NaN to index 0, a voxel of
+// every volume, where torch samples the zero padding.  Exact for |p| < 2^22; anything further out, inf and NaN included,
+// lands on an index no volume reaches.
+__device__ __forceinline__ int round_idx(float p)
+{
+    return __float_as_int(__fadd_rn(p, 12582912.f)) - 0x4B400000;
+}
+
+// The voxel grid_sample(mode='nearest', padding_mode='zeros') reads at (px,py,pz): its linear offset (64-bit), and
+// false when it lies in the zero padding.  2-D: D = 1, pz = 0.
+__device__ __forceinline__ bool nearest_offset(int D, int H, int W, float px, float py, float pz, long long &o)
+{
+    const int x = round_idx(px), y = round_idx(py), z = round_idx(pz);
+    o = ((long long)z * H + y) * W + x;
+    return (unsigned)x < (unsigned)W && (unsigned)y < (unsigned)H && (unsigned)z < (unsigned)D;
 }
 
 // the 8 corners of the cell with origin (x0,y0,z0), zero outside the volume: predicated loads, 64-bit offsets

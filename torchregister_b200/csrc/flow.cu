@@ -24,18 +24,20 @@ __device__ __forceinline__ FlowAxes flow_axes(int D, int H, int W)
     a.x = axis_map(W); a.y = axis_map(H); a.z = axis_map(D > 1 ? D : 2);
     return a;
 }
-template <int NDIM>
+// DEVICE_GRID: the reference's grid as torch forms it on a CUDA device (flow_pos_rcp), else as on the CPU (flow_pos)
+template <int NDIM, bool DEVICE_GRID = false>
 __device__ __forceinline__ void flow_position(const float *__restrict__ flow, size_t vol, size_t idx, int x, int y, int z,
                                               const FlowAxes &ax, float &px, float &py, float &pz)
 {
+    const auto pos = [](const AxisMap &m, int i, float f) { return DEVICE_GRID ? flow_pos_rcp(m, i, f) : flow_pos(m, i, f); };
     if (NDIM == 3) {
-        pz = flow_pos(ax.z, z, ld_stream_f(flow + idx));
-        py = flow_pos(ax.y, y, ld_stream_f(flow + vol + idx));
-        px = flow_pos(ax.x, x, ld_stream_f(flow + 2 * vol + idx));
+        pz = pos(ax.z, z, ld_stream_f(flow + idx));
+        py = pos(ax.y, y, ld_stream_f(flow + vol + idx));
+        px = pos(ax.x, x, ld_stream_f(flow + 2 * vol + idx));
     } else {
         pz = 0.f;
-        py = flow_pos(ax.y, y, ld_stream_f(flow + idx));
-        px = flow_pos(ax.x, x, ld_stream_f(flow + vol + idx));
+        py = pos(ax.y, y, ld_stream_f(flow + idx));
+        px = pos(ax.x, x, ld_stream_f(flow + vol + idx));
     }
 }
 
@@ -50,6 +52,23 @@ __global__ void __launch_bounds__(256, 4) warp_flow_kernel(const float *__restri
         flow_position<NDIM>(flow, vol, idx, x, y, z, ax, px, py, pz);
         for (int c = 0; c < n_channels; ++c)
             out[(size_t)c * vol + idx] = sample_zero_pad<NDIM, false>(src + (size_t)c * vol, D, H, W, px, py, pz).val;
+    });
+}
+
+// grid_sample(mode='nearest', align_corners=True) on the reference's grid as the device forms it: flow_position<.., true>
+// reproduces that fp32 grid op for op and round_idx is torch's nearbyint, so the result is torch's on CUDA bit for bit
+template <int NDIM>
+__global__ void __launch_bounds__(256, 4) warp_flow_nearest_kernel(const float *__restrict__ src, const float *__restrict__ flow,
+                                                                 float *__restrict__ out, int n_channels, int D, int H, int W)
+{
+    const size_t vol = (size_t)(NDIM == 3 ? D : 1) * H * W;
+    const FlowAxes ax = flow_axes(D, H, W);
+    for_each_voxel<2>(NDIM == 3 ? D : 1, H, W, [&](size_t idx, int x, int y, int z) {
+        float px, py, pz;
+        flow_position<NDIM, true>(flow, vol, idx, x, y, z, ax, px, py, pz);
+        long long o;
+        const bool v = nearest_offset(NDIM == 3 ? D : 1, H, W, px, py, pz, o);
+        for (int c = 0; c < n_channels; ++c) out[(size_t)c * vol + idx] = v ? __ldg(src + (size_t)c * vol + o) : 0.f;
     });
 }
 
@@ -306,6 +325,12 @@ extern "C" size_t trb_flow_workspace_bytes(void) { return (size_t)(8 + kFlowMaxB
 extern "C" int trb_warp_flow(int ndim, const float *src_dev, const float *flow_dev, float *out_dev, int n_channels,
                              int D, int H, int W, void *stream)
 {
+    return trb_warp_flow_ex(ndim, src_dev, flow_dev, out_dev, n_channels, D, H, W, 0, stream);
+}
+
+extern "C" int trb_warp_flow_ex(int ndim, const float *src_dev, const float *flow_dev, float *out_dev, int n_channels,
+                                int D, int H, int W, int flags, void *stream)
+{
     int rc = validate_flow(ndim, D, H, W);
     if (rc) return rc;
     if (!src_dev || !flow_dev || !out_dev || n_channels < 1) { set_error("null pointer / n_channels"); return TRB_ERR_ARG; }
@@ -313,8 +338,14 @@ extern "C" int trb_warp_flow(int ndim, const float *src_dev, const float *flow_d
     unsigned g;
     if ((rc = flow_grid(vol, g))) return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    if (ndim == 3) warp_flow_kernel<3><<<g, 256, 0, s>>>(src_dev, flow_dev, out_dev, n_channels, D, H, W);
-    else warp_flow_kernel<2><<<g, 256, 0, s>>>(src_dev, flow_dev, out_dev, n_channels, 1, H, W);
+    if (flags & TRB_FLAG_NEAREST) {
+        if (ndim == 3) warp_flow_nearest_kernel<3><<<g, 256, 0, s>>>(src_dev, flow_dev, out_dev, n_channels, D, H, W);
+        else warp_flow_nearest_kernel<2><<<g, 256, 0, s>>>(src_dev, flow_dev, out_dev, n_channels, 1, H, W);
+    } else if (ndim == 3) {
+        warp_flow_kernel<3><<<g, 256, 0, s>>>(src_dev, flow_dev, out_dev, n_channels, D, H, W);
+    } else {
+        warp_flow_kernel<2><<<g, 256, 0, s>>>(src_dev, flow_dev, out_dev, n_channels, 1, H, W);
+    }
     return check_cuda(cudaGetLastError(), "warp_flow");
 }
 

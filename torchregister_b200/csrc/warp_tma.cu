@@ -33,8 +33,10 @@ struct WarpParams {
     int n_channels;
 };
 
-__global__ void __launch_bounds__(kWarpThreads, 1)
-warp_affine_tma_kernel(const WarpParams wp, const __grid_constant__ CUtensorMap map_mov)
+// NEAREST: grid_sample(mode='nearest'): same producer, box bound, ring and tile walk; each consumer reads the one staged
+// voxel at the rounded coordinate (box_nearest), tiles off the box one predicated global load (nearest_offset)
+template <bool NEAREST>
+__device__ __forceinline__ void warp_affine_tma_body(const WarpParams &wp, const CUtensorMap &map_mov)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem_raw + kWOffBars);
@@ -171,7 +173,27 @@ warp_affine_tma_kernel(const WarpParams wp, const __grid_constant__ CUtensorMap 
         const size_t HW = (size_t)H * W;
         if (valid) {
             float *o = dst + (size_t)m.z0 * HW;
-            if ((m.flags & kWFits) && m.nz == TZ) {
+            if constexpr (NEAREST) {
+                if (m.flags & kWFits) {
+                    // voxel pairs (z, z + 1) as in the bilinear path; an odd tail's second voxel lies inside the
+                    // bounded footprint (the bound covers all TZ slices of a tile) and is not stored
+                    float2 zf = make_float2(m.zf0, m.zf0 + 1.f);
+                    for (int zz = 0; zz < m.nz; zz += 2) {
+                        const float2 tb = box_nearest<kBX, kBY>(m.Mrel, __ffma2_rn(f2(sz[0]), zf, f2(pxy[0])),
+                                                                __ffma2_rn(f2(sz[1]), zf, f2(pxy[1])), __ffma2_rn(f2(sz[2]), zf, f2(pxy[2])));
+                        __stcs(o + (size_t)zz * HW, lds_f<0>(cell_addr(box_addr, tb.x)));
+                        if (zz + 1 < m.nz) __stcs(o + (size_t)(zz + 1) * HW, lds_f<0>(cell_addr(box_addr, tb.y)));
+                        zf = __fadd2_rn(zf, f2(2.f));
+                    }
+                } else {
+                    for (int zz = 0; zz < m.nz; ++zz) {
+                        const float zf = m.zf0 + (float)zz;
+                        long long off;
+                        const bool v = nearest_offset(D, H, W, fmaf(sz[0], zf, pxy[0]), fmaf(sz[1], zf, pxy[1]), fmaf(sz[2], zf, pxy[2]), off);
+                        __stcs(o + (size_t)zz * HW, v ? __ldg(mov + off) : 0.f);
+                    }
+                }
+            } else if ((m.flags & kWFits) && m.nz == TZ) {
                 float2 zf = make_float2(m.zf0, m.zf0 + 1.f);
 #pragma unroll
                 for (int j = 0; j < TZ / 2; ++j) {
@@ -205,6 +227,18 @@ warp_affine_tma_kernel(const WarpParams wp, const __grid_constant__ CUtensorMap 
     }
 }
 
+__global__ void __launch_bounds__(kWarpThreads, 1)
+warp_affine_tma_kernel(const WarpParams wp, const __grid_constant__ CUtensorMap map_mov)
+{
+    warp_affine_tma_body<false>(wp, map_mov);
+}
+
+__global__ void __launch_bounds__(kWarpThreads, 1)
+warp_affine_nearest_tma_kernel(const WarpParams wp, const __grid_constant__ CUtensorMap map_mov)
+{
+    warp_affine_tma_body<true>(wp, map_mov);
+}
+
 bool warp_tma_eligible(const float *moving, const float *out, int n_items, long long vol, int D, int H, int W)
 {
     if (W % 4 != 0 || W < TX || H < TY || D < 1) return false;
@@ -216,7 +250,7 @@ bool warp_tma_eligible(const float *moving, const float *out, int n_items, long 
 
 // all (pair, channel) volumes of a batch in one launch; theta_dev: [n_pairs][12]
 int launch_warp_affine_tma(const float *moving, float *out, int n_pairs, int n_channels, int D, int H, int W,
-                           const float *theta_dev, const float *xb, const float *yb, cudaStream_t stream)
+                           const float *theta_dev, const float *xb, const float *yb, bool nearest, cudaStream_t stream)
 {
     const int n_items = n_pairs * n_channels;
     const long long vol = (long long)D * H * W;
@@ -239,9 +273,10 @@ int launch_warp_affine_tma(const float *moving, float *out, int n_pairs, int n_c
     const int grid = (int)grid_ll;
     wp.t.full_rounds = (int)(total_cols / grid);
     wp.t.tail_tiles = (total_cols - (long long)wp.t.full_rounds * grid) * wp.t.tiles_z;
-    cudaError_t e = cudaFuncSetAttribute(warp_affine_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWSmem);
+    const auto kernel = nearest ? warp_affine_nearest_tma_kernel : warp_affine_tma_kernel;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWSmem);
     if (e != cudaSuccess) return check_cuda(e, "cudaFuncSetAttribute(warp_affine_tma)");
-    warp_affine_tma_kernel<<<grid, kWarpThreads, kWSmem, stream>>>(wp, map_mov);
+    kernel<<<grid, kWarpThreads, kWSmem, stream>>>(wp, map_mov);
     return check_cuda(cudaGetLastError(), "warp_affine_tma");
 }
 

@@ -300,13 +300,28 @@ class AffineProblem:
         return self.loss_log[:, : self.epoch]
 
 
+TRB_FLAG_NEAREST = 8
+
+
+def _mode_flag(mode: str) -> int:
+    """Sampling mode of the forward warps -> C-ABI flag: 'bilinear' (the reference's) or 'nearest' (label maps)."""
+    if mode == 'bilinear':
+        return 0
+    if mode == 'nearest':
+        return TRB_FLAG_NEAREST
+    raise ValueError("mode must be 'bilinear' or 'nearest' (got %r)" % (mode,))
+
+
 def warp_affine(theta: torch.Tensor, moving: torch.Tensor, out: Optional[torch.Tensor] = None,
-                large_rotation: bool = False) -> torch.Tensor:
+                large_rotation: bool = False, *, mode: str = 'bilinear') -> torch.Tensor:
     """out[n, c] = grid_sample(moving[n, c], affine_grid(theta[n])), align_corners=False, zeros padding (reference
     get_affine_warp, warpings.py:18-26).  theta: 12|6 values per pair; moving [N,C,...] with N pairs (N == 1 is the
     reference's case, N > 1 the batch extension: every pair its own theta, ONE launch for all pairs and channels).
     `out`: optional contiguous fp32 destination of moving's shape.  `large_rotation`: theta is known to rotate by more
-    than a few degrees (3-D: take the gather kernel instead of the TMA-staged one; same values either way)."""
+    than a few degrees (3-D: take the gather kernel instead of the TMA-staged one; same values either way).
+    `mode='nearest'`: grid_sample(mode='nearest') for label maps — the source coordinate rounded half to even, so only
+    values of `moving` and 0 appear in the output (labels travel as fp32, exact up to 2^24)."""
+    flag = _mode_flag(mode)
     require_cuda(moving, "moving")
     ndim, D, H, W = _vol_dims(moving)
     lib = _lib.load()
@@ -327,8 +342,8 @@ def warp_affine(theta: torch.Tensor, moving: torch.Tensor, out: Optional[torch.T
     zb = base_coords(D, dev) if ndim == 3 else None
     with torch.cuda.device(dev):
         check(lib.trb_warp_affine_batch(ndim, src.data_ptr(), out.data_ptr(), n, int(src.shape[1]), D, H, W, th.data_ptr(),
-                                        xb.data_ptr(), yb.data_ptr(), _ptr(zb), 1 if large_rotation else 0, _stream(dev)),
-              "warp_affine")
+                                        xb.data_ptr(), yb.data_ptr(), _ptr(zb), (1 if large_rotation else 0) | flag,
+                                        _stream(dev)), "warp_affine")
     return out
 
 
@@ -422,16 +437,18 @@ def _check_flow(src: torch.Tensor, flow: torch.Tensor):
     return ndim, D, H, W
 
 
-def warp_flow(src: torch.Tensor, flow: torch.Tensor) -> torch.Tensor:
-    """SpatialTransformer.forward (reference utils.py:350-365), all channels of `src`."""
+def warp_flow(src: torch.Tensor, flow: torch.Tensor, *, mode: str = 'bilinear') -> torch.Tensor:
+    """SpatialTransformer.forward (reference utils.py:350-365), all channels of `src`.  `mode='nearest'`:
+    grid_sample(mode='nearest', align_corners=True) on the reference's grid, bit for bit (label maps)."""
+    flag = _mode_flag(mode)
     ndim, D, H, W = _check_flow(src, flow)
     lib = _lib.load()
     dev = src.device
     s, f = src.detach().contiguous(), flow.detach().contiguous()
     out = torch.empty_like(s)
     with torch.cuda.device(dev):
-        check(lib.trb_warp_flow(ndim, s.data_ptr(), f.data_ptr(), out.data_ptr(), int(s.shape[1]), D, H, W,
-                                _stream(dev)), "warp_flow")
+        check(lib.trb_warp_flow_ex(ndim, s.data_ptr(), f.data_ptr(), out.data_ptr(), int(s.shape[1]), D, H, W, flag,
+                                   _stream(dev)), "warp_flow")
     return out
 
 

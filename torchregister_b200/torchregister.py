@@ -106,11 +106,13 @@ class Register():
             self.losses = probs[0].losses[0] if moving.shape[0] == 1 else probs[0].losses   # device tensor(s): loss log
             self._last_problem = probs[0]             # final theta / params / best theta of the run (device state)
 
-    def __call__(self, moving):
+    def __call__(self, moving, *, mode='bilinear'):
         '''
         Warp `moving` [1,c,...] with the deformation found by `optim` (reference torchregister.py:108-129).
+        `mode` (keyword-only extension): 'bilinear' (the reference's) or 'nearest', for label maps such as a
+        segmentation or an atlas — only values of `moving` and 0 appear in the result.
         '''
         moving = moving.to(device=self.device, dtype=__import__('torch').float32)
         if self.mode == 'flow':
-            return self.warp(moving)                 # all channels in one launch
-        return self.warp(self.theta, moving)
+            return self.warp(moving, mode=mode)      # all channels in one launch
+        return self.warp(self.theta, moving, mode=mode)

@@ -295,33 +295,39 @@ class Regressor(nn.Module):
 # --------------------------------------------------------------------------- #
 class _WarpFlowFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, src, flow):
+    def forward(ctx, src, flow, mode='bilinear'):
         ctx.save_for_backward(src, flow)
-        return TF.warp_flow(src, flow)
+        ctx.mode = mode
+        return TF.warp_flow(src, flow, mode=mode)
 
     @staticmethod
     def backward(ctx, grad_out):
         src, flow = ctx.saved_tensors
+        if ctx.mode == 'nearest':
+            # a nearest sample is piecewise constant in the position: d/d flow is 0 (torch's nearest grid_sample gives
+            # the grid the same zero gradient)
+            return None, torch.zeros_like(flow) if ctx.needs_input_grad[1] else None, None
         if src.shape[1] != 1:
             raise NotImplementedError("gradient of the flow warp is implemented for single-channel src")
         dflow = TF.warp_flow_vjp(src, flow, grad_out.contiguous()) if ctx.needs_input_grad[1] else None
-        return None, dflow       # no gradient to `src`: the moving image is constant on this path
+        return None, dflow, None       # no gradient to `src`: the moving image is constant on this path
 
 
 class SpatialTransformer(nn.Module):
     """N-D spatial transformer: samples `src` at voxel index + flow (voxel units, channel i
-    displaces spatial axis i), bilinear, zeros padding (reference utils.py:333-365).
+    displaces spatial axis i), zeros padding (reference utils.py:333-365), bilinear or nearest
+    (grid_sample's modes; 'nearest' carries label maps and gives the flow a zero gradient).
     The identity index grid the reference keeps as a buffer is computed in the kernel."""
 
     def __init__(self, size, mode='bilinear'):
         super().__init__()
-        if mode != 'bilinear':
-            raise NotImplementedError("only mode='bilinear' (the mode Register uses, torchregister.py:72-79)")
+        if mode not in ('bilinear', 'nearest'):
+            raise NotImplementedError("mode must be 'bilinear' or 'nearest' (got %r)" % (mode,))
         self.mode = mode
         self.size = tuple(int(s) for s in size)
 
     def forward(self, src, flow):
-        return _WarpFlowFn.apply(src, flow)
+        return _WarpFlowFn.apply(src, flow, self.mode)
 
 
 # --------------------------------------------------------------------------- #

@@ -40,11 +40,15 @@ class _AffineWarpFn(torch.autograd.Function):
         return dth, None
 
 
-def get_affine_warp(theta, moving):
+def get_affine_warp(theta, moving, *, mode='bilinear'):
     """warped = grid_sample(moving, affine_grid(theta), bilinear, zeros, align_corners=False)
     (reference warpings.py:18-26).  theta: [1,2,3] / [1,3,4] or flat [*,6] / [*,12].
     One fused kernel, no materialised grid; differentiable w.r.t. theta.  EXTENSION: a batch
-    moving [N,C,...] with theta [N,nd,nd+1] is warped pair-wise (the reference supports N == 1 only)."""
+    moving [N,C,...] with theta [N,nd,nd+1] is warped pair-wise (the reference supports N == 1 only).
+    EXTENSION `mode='nearest'` (keyword-only): grid_sample(mode='nearest') for label maps.  Its output carries no
+    autograd graph: a nearest warp is piecewise constant in theta, so its gradient is zero almost everywhere."""
+    if mode != 'bilinear':
+        return TF.warp_affine(theta, moving, mode=mode)
     if moving.shape[0] > 1:
         nd = moving.dim() - 2
         th = theta.reshape(moving.shape[0], nd, nd + 1)
@@ -291,6 +295,11 @@ class flow_register(nn.Module):
     def __init__(self, img_size, mode='bilinear', in_c=1, n=1,
                  criterions=None, weights=[0.33, 0.33, 0.33], lr=1E-3, max_epochs=2000, stop_crit=1E-4):
         super().__init__()
+        if mode != 'bilinear':
+            # the optimisation runs through the fused bilinear node, and a nearest warp would give the U-Net no gradient;
+            # label maps are carried afterwards with deform(x, mode='nearest')
+            raise NotImplementedError("flow_register trains with mode='bilinear' only (got %r); warp label maps with "
+                                      "deform(x, mode='nearest') after optimize" % (mode,))
         self.model = Attention_UNet(img_size, mode, in_c=in_c, n=n)
         self.flow = None
         self.warp = None
@@ -354,9 +363,10 @@ class flow_register(nn.Module):
         if debug:
             print('Optimization ended with status: %s' % message)
 
-    def deform(self, x):
-        """Warp `x` with the flow of the last forward pass (reference warpings.py:238-242)."""
-        return TF.warp_flow(x, self.flow.detach())
+    def deform(self, x, *, mode='bilinear'):
+        """Warp `x` with the flow of the last forward pass (reference warpings.py:238-242).  EXTENSION `mode='nearest'`
+        (keyword-only): nearest-neighbour sampling for label maps."""
+        return TF.warp_flow(x, self.flow.detach(), mode=mode)
 
 
 class direct_flow_register:
@@ -411,5 +421,6 @@ class direct_flow_register:
         if debug:
             print('Optimization ended with status: %s' % message)
 
-    def deform(self, x):
-        return TF.warp_flow(x, self.flow)
+    def deform(self, x, *, mode='bilinear'):
+        """Warp `x` with the optimised flow; `mode='nearest'` for label maps."""
+        return TF.warp_flow(x, self.flow, mode=mode)
