@@ -212,7 +212,8 @@ int trb_warp_affine(int ndim, const float *moving_dev, float *out_dev, int n_cha
  * [n_pairs][12|6], ONE launch.  3-D shapes with W % 4 == 0, W >= 32, H >= 16 take the TMA-staged kernel (csrc/warp_tma.cu);
  * flags: TRB_FLAG_LARGE_ROTATION = theta is known to rotate by more than a few degrees (gather kernel instead);
  * TRB_FLAG_NEAREST = grid_sample(mode='nearest'): the source coordinate rounded half to even, zero outside the volume,
- * so only input values and 0 appear in out (label maps).  Same path selection with or without it. */
+ * so only input values and 0 appear in out (label maps).  Same path selection with or without it.  The nearest kernels
+ * need every spatial axis <= 2^22 = 4194304 voxels (TRB_ERR_UNSUPPORTED otherwise); the bilinear ones do not. */
 int trb_warp_affine_batch(int ndim, const float *moving_dev, float *out_dev, int n_pairs, int n_channels,
                           int D, int H, int W, const float *theta_dev,
                           const float *xb_dev, const float *yb_dev, const float *zb_dev, int flags, void *stream);
@@ -232,7 +233,10 @@ int trb_warp_affine_vjp_ex(int ndim, const float *moving_dev, const float *gout_
 
 /* ---- flow field ----------------------------------------------------------- */
 /* flow layout [ndim][D][H][W] fp32 in voxel units, channel i displaces spatial
- * axis i (0 = D (3-D) or H (2-D)), the SpatialTransformer convention utils.py:350-365. */
+ * axis i (0 = D (3-D) or H (2-D)), the SpatialTransformer convention utils.py:350-365.
+ * The calls below that sample a volume (every one but trb_flow_jacobian) need every spatial axis >= 2,
+ * D*H*W < 2^31 (TRB_ERR_ARG otherwise) and every axis <= 2^22 = 4194304 voxels: their kernels take floor and rint with
+ * a 1.5*2^23 add, which indexes exactly only up to there (TRB_ERR_UNSUPPORTED otherwise). */
 
 size_t trb_flow_workspace_bytes(void);
 
@@ -276,7 +280,8 @@ int trb_flow_loss_grad(int ndim, const float *moving_dev, const float *target_de
  * feat_dev: the decoder output [C][fd][fh][fw] (C <= 8, un-padded); w_dev [ndim][C], b_dev [ndim]: the 1x1 `out`
  * convolution (device memory: the module's parameters as they are).  forward: writes flow_out_dev [ndim][D][H][W] (= Register.theta) and *loss_dev, leaves the loss
  * coefficients in the workspace; backward (same workspace, after forward): dfeat_dev [C][fd][fh][fw] = d loss / d feat,
- * dwb_dev[ndim*C + ndim] = d loss / d W, d loss / d b.  d loss / d flow is never written. */
+ * dwb_dev[ndim*C + ndim] = d loss / d W, d loss / d b.  d loss / d flow is never written.  Both calls refuse C > 8
+ * (TRB_ERR_UNSUPPORTED) and a feature map larger than the volume on some axis (TRB_ERR_ARG). */
 int trb_flow_head_forward(int ndim, const float *moving_dev, const float *target_dev, const float *feat_dev, int C,
                           int fd, int fh, int fw, const float *w_dev, const float *b_dev, int D, int H, int W,
                           float w_mse, float w_ncc, float *loss_dev, float *flow_out_dev,
@@ -293,6 +298,7 @@ int trb_flow_head_backward(int ndim, const float *moving_dev, const float *targe
  * Slab form (one volume sharded over GPUs by z): target/flow/adam arrays hold slices [z_off, z_off+Ds),
  * `moving` is the whole volume, halo_lo/halo_hi are the neighbouring ranks' flow slices z_off-1 and
  * z_off+Ds ([ndim][H][W]; NULL at the volume boundary).  A single GPU passes z_off=0, Ds=D, no halos.
+ * Every spatial axis must be <= 2^22 = 4194304 voxels, as for the flow calls above (TRB_ERR_UNSUPPORTED otherwise).
  * moments6: sum t, sum w, sum t^2, sum w^2, sum t*w, smooth (fp64, overwritten by stats). */
 size_t trb_flow_direct_workspace_bytes(void);
 

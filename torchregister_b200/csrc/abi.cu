@@ -36,6 +36,14 @@ int sm_count(int &n)
     return rc;
 }
 
+int check_fast_floor_axes(int ndim, int D, int H, int W)
+{
+    if (W <= kMaxFastFloorAxis && H <= kMaxFastFloorAxis && (ndim != 3 || D <= kMaxFastFloorAxis)) return TRB_OK;
+    set_error("every spatial axis must be at most 2^22 = %d voxels long (got %dx%dx%d): the sampling kernels' fast floor "
+              "indexes exactly only up to there", kMaxFastFloorAxis, ndim == 3 ? D : 1, H, W);
+    return TRB_ERR_UNSUPPORTED;
+}
+
 }  // namespace trb
 
 extern "C" int trb_abi_version(void) { return TRB_ABI_VERSION; }

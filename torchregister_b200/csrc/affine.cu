@@ -698,6 +698,9 @@ extern "C" int trb_warp_affine_batch(int ndim, const float *moving_dev, float *o
 {
     int rc = validate_common(ndim, n_pairs, D, H, W);
     if (rc) return rc;
+    // the nearest kernels round through round_idx; the bilinear gather kernels floor with floorf and take any axis (the
+    // TMA-staged ones are only eligible for axes far below the limit)
+    if ((flags & TRB_FLAG_NEAREST) && (rc = check_fast_floor_axes(ndim, D, H, W))) return rc;
     if (!moving_dev || !out_dev || !theta_dev || !xb_dev || !yb_dev || (ndim == 3 && !zb_dev) || n_channels < 1) {
         set_error("null pointer / n_channels"); return TRB_ERR_ARG;
     }

@@ -471,7 +471,8 @@ bool tma_path_eligible(int ndim, const AffineParams &a, int n_pairs)
     if (((uintptr_t)a.moving & 15) || ((uintptr_t)a.target & 15)) return false;
     if (n_pairs > 1 && (a.pair_stride % 4 != 0)) return false;
     if (n_pairs > kMaxTmaPairs) return false;
-    // fp32 index trick range: |x + BX*y + BX*BY*z| < 2^22 with some headroom
+    // fp32 index trick range: |x + BX*y + BX*BY*z| < 2^22 with some headroom.  It also keeps every axis far below
+    // kMaxFastFloorAxis, which the kMagic floor of the staged and clamped samples needs
     if ((double)a.W + (double)kBX * a.H + (double)kBX * kBY * a.D > 1.8e6) return false;
     {   // the pair-parity double buffer assumes a pair spans more tiles than the ring holds
         const long long tpp = (long long)((a.W + TX - 1) / TX) * ((a.H + TY - 1) / TY) * ((a.s_end - a.s_begin + TZ - 1) / TZ);

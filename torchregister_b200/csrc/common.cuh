@@ -18,6 +18,11 @@ void set_error(const char *fmt, ...);
 int check_cuda(cudaError_t e, const char *what);
 // SM count of the current device, queried once per device.  Returns TRB_OK, or the CUDA error with trb_last_error() set.
 int sm_count(int &n);
+// The longest spatial axis the 1.5*2^23 floor / rint below (floor_frac, round_idx, and kMagic in the TMA-staged
+// kernels) can index: TRB_ERR_UNSUPPORTED, with trb_last_error() naming the limit, when an axis of (D,) H, W is longer.
+// Every entry point whose kernels index a volume through them calls it.
+constexpr int kMaxFastFloorAxis = 1 << 22;
+int check_fast_floor_axes(int ndim, int D, int H, int W);
 
 // ---- loads ---------------------------------------------------------------
 __device__ __forceinline__ float ldg_f(const float *p) { return __ldg(p); }
@@ -192,8 +197,10 @@ __device__ __forceinline__ float flow_pos_rcp(const AxisMap &m, int i, float f)
 }
 
 // floor and fraction without the quarter-rate conversion pipe: adding 1.5*2^23 rounding down leaves floor(p) in the
-// low mantissa bits (exact for |p| < 2^22; anything further out — inf and NaN included — lands on an index no volume
-// reaches, i.e. on the zero padding).
+// low mantissa bits, exactly for |p| <= 2^22.  Further out the sum's spacing differs from 1 and the index is wrong, but it
+// is >= 2^22 or < -2^22 (inf and NaN included), so with every axis at most 2^22 voxels long (kMaxFastFloorAxis; hosts
+// refuse longer ones) such a position still lands on the zero padding.  On a longer axis it would read a wrong voxel
+// inside the volume: p = 4195304.25 gives index 4194804.
 __device__ __forceinline__ void floor_frac(float p, int &i0, float &t, float &fl)
 {
     const float m = __fadd_rd(p, 12582912.f);
@@ -210,7 +217,7 @@ __device__ __forceinline__ void floor_frac(float p, int &i0, float &t)
 // grid_sample(mode='nearest')'s source index: p rounded half to even, as torch's nearbyint does.  The same 1.5*2^23 add
 // as floor_frac, in round-to-nearest mode, rather than __float2int_rn: the conversion maps NaN to index 0, a voxel of
 // every volume, where torch samples the zero padding.  Exact for |p| < 2^22; anything further out, inf and NaN included,
-// lands on an index no volume reaches.
+// lands on an index >= 2^22 or < -2^22: the zero padding of any axis of at most kMaxFastFloorAxis voxels (see floor_frac).
 __device__ __forceinline__ int round_idx(float p)
 {
     return __float_as_int(__fadd_rn(p, 12582912.f)) - 0x4B400000;

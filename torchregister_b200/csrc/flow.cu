@@ -313,7 +313,7 @@ static int validate_flow(int ndim, int D, int H, int W)
     if (ndim != 2 && ndim != 3) { set_error("ndim must be 2 or 3 (got %d)", ndim); return TRB_ERR_ARG; }
     if (H < 2 || W < 2 || (ndim == 3 && D < 2)) { set_error("flow warp needs every axis >= 2 (got %dx%dx%d)", D, H, W); return TRB_ERR_ARG; }
     if ((unsigned long long)(ndim == 3 ? D : 1) * H * W >= (1ull << 31)) { set_error("flow kernels index volumes with 32 bits: D*H*W must stay below 2^31"); return TRB_ERR_ARG; }
-    return TRB_OK;
+    return check_fast_floor_axes(ndim, D, H, W);
 }
 
 }  // namespace trb
@@ -429,6 +429,7 @@ extern "C" int trb_flow_head_backward(int ndim, const float *moving_dev, const f
     if (rc) return rc;
     if (!moving_dev || !target_dev || !flow_dev || !feat_dev || !w_dev || !dfeat_dev || !dwb_dev) { set_error("null pointer"); return TRB_ERR_ARG; }
     if (C < 1 || C > kHeadMaxC) { set_error("the fused U-Net head handles 1..%d feature channels (got %d)", kHeadMaxC, C); return TRB_ERR_UNSUPPORTED; }
+    if (fw > W || fh > H || (ndim == 3 && fd > D) || fw < 1 || fh < 1 || fd < 1) { set_error("feature map larger than the volume"); return TRB_ERR_ARG; }
     if (!workspace_dev || workspace_bytes < trb_flow_workspace_bytes()) { set_error("workspace too small"); return TRB_ERR_WORKSPACE; }
     FlowHead h{};
     h.feat = feat_dev; h.C = C; h.fd = ndim == 3 ? fd : 1; h.fh = fh; h.fw = fw;

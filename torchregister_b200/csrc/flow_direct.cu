@@ -619,6 +619,7 @@ static int fill_direct(DirectParams &p, int ndim, const float *moving, const flo
 {
     if (ndim != 2 && ndim != 3) { set_error("ndim must be 2 or 3"); return TRB_ERR_ARG; }
     if (H < 2 || W < 2 || (ndim == 3 && D < 2)) { set_error("flow needs every axis >= 2"); return TRB_ERR_ARG; }
+    if (int rc = check_fast_floor_axes(ndim, D, H, W)) return rc;
     if (!moving || !target || !flow_in || !moments) { set_error("null pointer"); return TRB_ERR_ARG; }
     if ((unsigned long long)(ndim == 3 ? D : 1) * H * W >= (1ull << 31)) { set_error("flow kernels index volumes with 32 bits: D*H*W must stay below 2^31"); return TRB_ERR_ARG; }
     if (ndim == 3 && (z_off < 0 || Ds < 1 || z_off + Ds > D)) { set_error("bad slab [%d,%d) of %d", z_off, z_off + Ds, D); return TRB_ERR_ARG; }
@@ -665,6 +666,7 @@ extern "C" int trb_flow_direct_update(int ndim, const float *moving_dev, const f
 {
     DirectParams p{};
     if (ndim != 2 && ndim != 3) { set_error("ndim must be 2 or 3"); return TRB_ERR_ARG; }
+    if (int rc = check_fast_floor_axes(ndim, D, H, W)) return rc;
     if (!moving_dev || !target_slab_dev || !flow_in_slab_dev || !flow_out_slab_dev || !moments6_dev) { set_error("null pointer"); return TRB_ERR_ARG; }
     if (flow_in_slab_dev == flow_out_slab_dev) { set_error("update is out of place: flow_out must differ from flow_in"); return TRB_ERR_ARG; }
     if ((unsigned long long)(ndim == 3 ? D : 1) * H * W >= (1ull << 31)) { set_error("flow kernels index volumes with 32 bits: D*H*W must stay below 2^31"); return TRB_ERR_ARG; }

@@ -244,6 +244,7 @@ bool warp_tma_eligible(const float *moving, const float *out, int n_items, long 
     if (W % 4 != 0 || W < TX || H < TY || D < 1) return false;
     if (((uintptr_t)moving & 15) || ((uintptr_t)out & 3)) return false;
     if (n_items > 1 && (vol % 4 != 0)) return false;
+    // the staged-box index range; it also keeps every axis far below kMaxFastFloorAxis (the kMagic floor / rint)
     if ((double)W + (double)kBX * H + (double)kBX * kBY * D > 1.8e6) return false;
     return encode_fn() != nullptr;
 }
