@@ -261,6 +261,39 @@ int trb_warp_flow_ex(int ndim, const float *src_dev, const float *flow_dev, floa
 int trb_flow_jacobian(int ndim, const float *flow_dev, int D, int H, int W, float *det_out_dev, double *stats_out_dev,
                       void *workspace_dev, size_t workspace_bytes, void *stream);
 
+/* Transform algebra (csrc/transform.cu).  A flow u stands for phi_u(p) = p + u(p); trb_warp_flow samples at phi_u(p).
+ * trb_warp_affine samples at T(q) = M q + c, theta's map in voxel units (affine_grid(align_corners=False) un-normalised by
+ * grid_sample): with S_r the size along sampling coordinate r (0 = x/W, 1 = y/H, 2 = z/D),
+ *   M_rc = theta_rc S_r / S_c,   c_r = S_r/2 (theta_r,ndim + 1 - sum_c theta_rc (1 - 1/S_c)) - 1/2.
+ * The composed field w of "first, then second" satisfies warp_flow(m, w) = warp_flow(warp(m, first), second) up to the
+ * interpolation of the intermediate volume that it avoids.  first~ is the (bi|tri)linear interpolant of a flow with border
+ * padding: each coordinate clamped to [0, S-1] (grid_sample(padding_mode='border', align_corners=True) on voxel positions).
+ * N == 1, no gradients; the shape rules of the flow calls above (TRB_ERR_ARG, TRB_ERR_UNSUPPORTED).  An output that
+ * overlaps an input is refused (TRB_ERR_ARG).  A non-finite sample position p + u(p) gives NaN in every channel of its
+ * voxel; a NaN among the corners of a cell that is read propagates to that channel. */
+
+/* w = T_theta(p + u(p)) - p, evaluated as u + (M - I) q + c with q = p + u (fp32 per voxel; M - I and c formed in fp64 from
+ * theta_dev, ndim*(ndim+1) floats in device memory, read by the kernel: no host synchronisation).  Exact: T is affine.
+ * flow_dev NULL: u = 0 (the affine's own displacement, T(p) - p).  out_dev: [ndim][D][H][W]. */
+int trb_compose_affine_flow(int ndim, const float *theta_dev, const float *flow_dev, int D, int H, int W,
+                            float *out_dev, void *stream);
+/* w = u(p) + first~(p + u(p)), u = second_dev; all three [ndim][D][H][W]. */
+int trb_compose_flows(int ndim, const float *first_dev, const float *second_dev, int D, int H, int W,
+                      float *out_dev, void *stream);
+/* Inverse: v = the fixed point of v(p) = -u~(p + v(p)), so that phi_u(phi_v(p)) = p, iterated per voxel: v_0 = -u(p);
+ * iteration k evaluates r_k = |v_k + u~(p + v_k)|_inf and stops when r_k <= tol or k = max_iter - 1, else
+ * v_{k+1} = -u~(p + v_k).  The v_k whose residual was evaluated is written to inv_out_dev, so each voxel's residual is the
+ * one counted below.  The iteration converges where u~ is a contraction (Lipschitz constant < 1 in the inf-norm: a mild,
+ * fold-free flow); the call does not require it and reports what did not converge.  A voxel that meets a non-finite
+ * position or residual stops there with NaN in every channel.  max_iter in [1, 1000], tol (voxels) finite and > 0
+ * (TRB_ERR_ARG otherwise).  stats_out_dev (dev, TRB_INV_NSTATS doubles): n not converged (finite, r > tol), n non-finite,
+ * max r over the finite voxels (0 if none), sum over all voxels of the residual evaluations made (iterations started).
+ * Counts and sums in a fixed order: the same bits on every run.  workspace: trb_flow_workspace_bytes() (its ticket must
+ * be zero, as for the flow calls; the call leaves it so). */
+#define TRB_INV_NSTATS 4
+int trb_invert_flow(int ndim, const float *flow_dev, int D, int H, int W, int max_iter, float tol,
+                    float *inv_out_dev, double *stats_out_dev, void *workspace_dev, size_t workspace_bytes, void *stream);
+
 /* dflow = J^T gout for the warp above (autograd of utils.py:365 w.r.t. flow);
  * used when the caller supplies its own criterion (torchregister.py:71-73). */
 int trb_warp_flow_vjp(int ndim, const float *src_dev, const float *flow_dev, const float *gout_dev,

@@ -10,6 +10,7 @@ from .utils import *            # noqa: F401,F403   (mirrors TR/__init__.py:1-3 
 from .warpings import *         # noqa: F401,F403
 from .torchregister import Register   # noqa: F401
 from .metrics import jacobian_determinant, dice   # noqa: F401
-from . import functional, synth, metrics      # noqa: F401
+from .transforms import affine_to_flow, compose_flow, invert_flow   # noqa: F401
+from . import functional, synth, metrics, transforms      # noqa: F401
 
 __version__ = '0.1.0'

@@ -48,6 +48,9 @@ _SIGNATURES = {
     "trb_warp_flow_ex": (_i, [_i, c_fp, c_fp, c_fp, _i, _i, _i, _i, _i, c_fp]),
     "trb_warp_flow_vjp": (_i, [_i, c_fp, c_fp, c_fp, c_fp, _i, _i, _i, c_fp]),
     "trb_flow_jacobian": (_i, [_i, c_fp, _i, _i, _i, c_fp, c_fp, c_fp, _sz, c_fp]),
+    "trb_compose_affine_flow": (_i, [_i, c_fp, c_fp, _i, _i, _i, c_fp, c_fp]),
+    "trb_compose_flows": (_i, [_i, c_fp, c_fp, _i, _i, _i, c_fp, c_fp]),
+    "trb_invert_flow": (_i, [_i, c_fp, _i, _i, _i, _i, _f, c_fp, c_fp, c_fp, _sz, c_fp]),
     "trb_flow_loss_grad": (_i, [_i, c_fp, c_fp, c_fp, _i, _i, _i, _f, _f, c_fp, c_fp, c_fp, c_fp, _sz, c_fp]),
     "trb_flow_head_forward": (_i, [_i, c_fp, c_fp, c_fp, _i, _i, _i, _i, c_fp, c_fp, _i, _i, _i,
                                    _f, _f, c_fp, c_fp, c_fp, _sz, c_fp]),

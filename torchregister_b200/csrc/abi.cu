@@ -44,6 +44,26 @@ int check_fast_floor_axes(int ndim, int D, int H, int W)
     return TRB_ERR_UNSUPPORTED;
 }
 
+int validate_flow(int ndim, int D, int H, int W)
+{
+    if (ndim != 2 && ndim != 3) { set_error("ndim must be 2 or 3 (got %d)", ndim); return TRB_ERR_ARG; }
+    if (H < 2 || W < 2 || (ndim == 3 && D < 2)) { set_error("flow warp needs every axis >= 2 (got %dx%dx%d)", D, H, W); return TRB_ERR_ARG; }
+    if ((unsigned long long)(ndim == 3 ? D : 1) * H * W >= (1ull << 31)) { set_error("flow kernels index volumes with 32 bits: D*H*W must stay below 2^31"); return TRB_ERR_ARG; }
+    return check_fast_floor_axes(ndim, D, H, W);
+}
+
+int flow_grid(size_t vol, unsigned &grid)
+{
+    int sms;
+    if (int rc = sm_count(sms)) return rc;
+    size_t nb = (vol + 255) / 256;      // enough CTAs for every SM to hold 8; each strides over row pairs
+    const size_t cap = (size_t)sms * 8;
+    if (nb > cap) nb = cap;
+    if (nb > kFlowMaxBlocks) nb = kFlowMaxBlocks;
+    grid = (unsigned)(nb < 1 ? 1 : nb);
+    return TRB_OK;
+}
+
 }  // namespace trb
 
 extern "C" int trb_abi_version(void) { return TRB_ABI_VERSION; }

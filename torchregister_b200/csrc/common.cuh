@@ -23,6 +23,13 @@ int sm_count(int &n);
 // Every entry point whose kernels index a volume through them calls it.
 constexpr int kMaxFastFloorAxis = 1 << 22;
 int check_fast_floor_axes(int ndim, int D, int H, int W);
+// The shape rules of every call that samples a flow-layout field (flow.cu, transform.cu): ndim 2 or 3, every spatial
+// axis >= 2, D*H*W < 2^31 (TRB_ERR_ARG), and check_fast_floor_axes.  2-D callers pass any D: it is not read.
+int validate_flow(int ndim, int D, int H, int W);
+// Grid of the one-thread-per-voxel flow kernels (for_each_voxel): enough CTAs for every SM to hold 8, at most
+// kFlowMaxBlocks (the partial rows of the flow workspace, trb_flow_workspace_bytes).
+constexpr int kFlowMaxBlocks = 2048;
+int flow_grid(size_t vol, unsigned &grid);
 
 // ---- loads ---------------------------------------------------------------
 __device__ __forceinline__ float ldg_f(const float *p) { return __ldg(p); }

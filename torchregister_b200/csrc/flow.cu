@@ -96,7 +96,6 @@ __global__ void __launch_bounds__(256) warp_flow_vjp_kernel(const float *__restr
 }
 
 // workspace layout (doubles): [0..3] cw, ct, c0, loss ; [4] ticket (as unsigned) ; [8..] partials[blocks][5]
-constexpr int kFlowMaxBlocks = 2048;
 
 template <int NDIM>
 __global__ void __launch_bounds__(256) flow_stats_kernel(const float *__restrict__ moving, const float *__restrict__ target,
@@ -294,26 +293,6 @@ __global__ void __launch_bounds__(256) flow_head_backward_kernel(const float *__
     const int i = threadIdx.x, a = i / (kHeadMaxC + 1), c = i - a * (kHeadMaxC + 1);
     if (c < h.C) dwb_out[a * h.C + c] = (float)red[0][i];
     else if (c == kHeadMaxC) dwb_out[NDIM * h.C + a] = (float)red[0][i];
-}
-
-static int flow_grid(size_t vol, unsigned &grid)
-{
-    int sms;
-    if (int rc = sm_count(sms)) return rc;
-    size_t nb = (vol + 255) / 256;      // enough CTAs for every SM to hold 8; each strides over row pairs
-    const size_t cap = (size_t)sms * 8;
-    if (nb > cap) nb = cap;
-    if (nb > kFlowMaxBlocks) nb = kFlowMaxBlocks;
-    grid = (unsigned)(nb < 1 ? 1 : nb);
-    return TRB_OK;
-}
-
-static int validate_flow(int ndim, int D, int H, int W)
-{
-    if (ndim != 2 && ndim != 3) { set_error("ndim must be 2 or 3 (got %d)", ndim); return TRB_ERR_ARG; }
-    if (H < 2 || W < 2 || (ndim == 3 && D < 2)) { set_error("flow warp needs every axis >= 2 (got %dx%dx%d)", D, H, W); return TRB_ERR_ARG; }
-    if ((unsigned long long)(ndim == 3 ? D : 1) * H * W >= (1ull << 31)) { set_error("flow kernels index volumes with 32 bits: D*H*W must stay below 2^31"); return TRB_ERR_ARG; }
-    return check_fast_floor_axes(ndim, D, H, W);
 }
 
 }  // namespace trb
