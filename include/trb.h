@@ -391,6 +391,47 @@ int trb_flow_direct_finish(const double *moments6_dev, int D, int H, int W, floa
                            float smooth_lambda, float *loss_log_dev, int epochs_done,
                            void *workspace_dev, size_t workspace_bytes, void *stream);
 
+/* The update pass of the direct-flow epoch driven by local NCC (single GPU, whole volume): one epoch is
+ * trb_flow_direct_stats -> trb_warp_flow (J) -> trb_lncc_forward -> trb_lncc_backward (resid = dL/dJ, its pointwise
+ * MSE / NCC terms from moments6) -> this call.  It recomputes the sample gradient G at flow_in and applies
+ * resid * G + lambda * (smoothness stencil) with SGD or Adam, as trb_flow_direct_update; flow_out must not overlap
+ * flow_in or resid (TRB_ERR_ARG).  loss_log_dev[epoch] (nullable) receives the loss of flow_in:
+ * w_mse*MSE + w_ncc*100*(1-NCC) (from moments6_dev) + w_lncc * lncc_stats_dev[1] + lambda * moments6_dev[5].
+ * Shape rules of trb_flow_direct_update with z_off = 0, Ds = D. */
+int trb_flow_direct_update_lncc(int ndim, const float *moving_dev, const float *flow_in_dev, float *flow_out_dev,
+                                const float *resid_dev, int D, int H, int W, const double *moments6_dev,
+                                const double *lncc_stats_dev, float w_mse, float w_ncc, float w_lncc,
+                                float smooth_lambda, float lr, int optimiser, float beta1, float beta2,
+                                float adam_eps, int step_index, float *adam_m_dev, float *adam_v_dev,
+                                float *loss_log_dev, int epoch, void *stream);
+
+/* ---- local normalised cross-correlation (csrc/lncc.cu) ------------------------------------------------------
+ * VoxelMorph's windowed NCC with the sign turned so that the loss is >= 0.  target I and warped J: fp32
+ * [N][D][H][W] (2-D: D ignored), N pairs that never share a window; win odd in [3, 15] (TRB_ERR_UNSUPPORTED
+ * otherwise); n = win^ndim; S_X the box sum of X over the window with zero padding (out-of-volume positions count
+ * as zeros, n stays fixed):
+ *   A = S_IJ - S_I S_J / n,  B = S_II - S_I^2 / n,  C = S_JJ - S_J^2 / n,  cc = A^2 / (B C + eps),
+ *   loss = 1 - (sum of cc over every voxel of every pair) / (N D H W).
+ * Shape rules: every axis >= 1, D*H*W < 2^31 (TRB_ERR_ARG) and every axis <= 2^22 (TRB_ERR_UNSUPPORTED).  An
+ * output that overlaps an input is refused (TRB_ERR_ARG).  Every sum is formed in a fixed order: the same bits on
+ * every run. */
+size_t trb_lncc_workspace_bytes(void);
+
+/* coef_dev: 3 N D H W floats, written as alpha, beta, gamma planes ([3][N][D][H][W]) with den = B C + eps,
+ * gamma = 2 A / den, beta = -A^2 B / den^2, alpha = -gamma S_I / n - 2 beta S_J / n (the derivatives of cc w.r.t.
+ * S_J, S_JJ, S_IJ).  stats_dev (dev, 2 doubles): sum of cc, loss.  eps finite and > 0.  workspace:
+ * trb_lncc_workspace_bytes() (its ticket must be zero, e.g. a zeroed buffer; the call leaves it so). */
+int trb_lncc_forward(int ndim, const float *target_dev, const float *warped_dev, int N, int D, int H, int W, int win,
+                     float eps, float *coef_dev, double *stats_dev, void *workspace_dev, size_t workspace_bytes,
+                     void *stream);
+
+/* grad_dev (N D H W floats) = scale * dloss/dJ = -(scale / (N D H W)) (box(alpha) + 2 J box(beta) + I box(gamma)),
+ * from the coef_dev of trb_lncc_forward on the same I, J and win.  With moments6_dev (N == 1 only; the layout of
+ * trb_flow_direct_stats), it adds the pointwise gradient of w_mse*MSE + w_ncc*100*(1-NCC): cw J + ct I + c0. */
+int trb_lncc_backward(int ndim, const float *target_dev, const float *warped_dev, const float *coef_dev, int N, int D,
+                      int H, int W, int win, float scale, const double *moments6_dev, float w_mse, float w_ncc,
+                      float *grad_dev, void *stream);
+
 /* ---- Edge3D pre-filter (SURVEY.md 8 f-4) --------------------------------------------------------------
  * Replaces utils.py:130-183 (Edge3D.__call__ with a pad that works): reflect padding, the nine 3x3x3 Sobel-type
  * cross-correlations of get_sobel_kernel3D (utils.py:82-127; passed as weights_host[9][27], HOST memory, (x,y,z) order),

@@ -67,6 +67,11 @@ _SIGNATURES = {
                                        c_fp, _sz, c_fp]),
     "trb_flow_direct_set_path": (None, [_i]),
     "trb_flow_direct_finish": (_i, [c_fp, _i, _i, _i, _f, _f, _f, c_fp, _i, c_fp, _sz, c_fp]),
+    "trb_flow_direct_update_lncc": (_i, [_i, c_fp, c_fp, c_fp, c_fp, _i, _i, _i, c_fp, c_fp, _f, _f, _f, _f, _f, _i,
+                                         _f, _f, _f, _i, c_fp, c_fp, c_fp, _i, c_fp]),
+    "trb_lncc_workspace_bytes": (_sz, []),
+    "trb_lncc_forward": (_i, [_i, c_fp, c_fp, _i, _i, _i, _i, _i, _f, c_fp, c_fp, c_fp, _sz, c_fp]),
+    "trb_lncc_backward": (_i, [_i, c_fp, c_fp, c_fp, _i, _i, _i, _i, _i, _f, c_fp, _f, _f, c_fp, c_fp]),
     "trb_affine_optim_peer": (_i, [c_fp, c_fp, _i, _i, _i, _i, _i, c_fp, c_fp, c_fp, _i, c_fp, c_fp, _i, _i, _i,
                                    _f, _f, _f, _i, _f, _f, _f, C.POINTER(C.c_void_p), _i, _i, C.c_ulonglong, c_fp, _sz, c_fp]),
     "trb_edge3d": (_i, [c_fp, c_fp, _i, _i, _i, _i, _i, C.POINTER(C.c_float), _f, _f, c_fp, c_fp, c_fp]),

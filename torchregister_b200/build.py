@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_lib")
 LIB_PATH = os.path.join(OUT_DIR, "libtrb_b200.so")
-SOURCES = ["abi.cu", "affine.cu", "affine_tma.cu", "affine_persist.cu", "warp_tma.cu", "edge.cu", "flow.cu", "flow_direct.cu", "jacobian.cu", "transform.cu", "nmi.cu", "nmi_src.cu", "instnorm.cu", "thinconv.cu"]
+SOURCES = ["abi.cu", "affine.cu", "affine_tma.cu", "affine_persist.cu", "warp_tma.cu", "edge.cu", "flow.cu", "flow_direct.cu", "jacobian.cu", "transform.cu", "lncc.cu", "nmi.cu", "nmi_src.cu", "instnorm.cu", "thinconv.cu"]
 # every header under csrc/ plus the public C header: editing any of them makes the library stale
 HEADERS = sorted(f for f in os.listdir(CSRC) if f.endswith((".cuh", ".h", ".inc"))) + [os.path.join("..", "..", "include", "trb.h")]
 

@@ -183,6 +183,72 @@ __global__ void __launch_bounds__(256) flow_direct_update_kernel(const DirectPar
     });
 }
 
+// The update pass of the LNCC epoch (lncc.cu): dL/dJ comes from an array (trb_lncc_backward, which already added the
+// pointwise MSE / NCC terms) instead of cw*w + ct*t + c0; the sample gradient G, the smoothness stencil and SGD / Adam
+// are those of flow_direct_update_kernel.  Whole volume only (z_off 0, Ds = D): LNCC is single-GPU.
+// loss_log[epoch] = similarity(moments) + w_lncc * lncc_stats[1] + lambda * moments[5], the loss of flow_in.
+template <int NDIM>
+__global__ void __launch_bounds__(256) flow_direct_update_lncc_kernel(const DirectParams p, const float *__restrict__ resid,
+                                                                      const double *__restrict__ lncc_stats, const float w_lncc)
+{
+    const int W = p.W, H = p.H, D = NDIM == 3 ? p.D : 1, Ds = NDIM == 3 ? p.Ds : 1;
+    const size_t HW = (size_t)H * W, slab = HW * Ds;
+    const AxisMap ax = axis_map(W), ay = axis_map(H), az = axis_map(D > 1 ? D : 2);
+    if (threadIdx.x == 0 && blockIdx.x == 0 && p.loss_log) {
+        const double n = (double)D * H * W;
+        const LossCoef lc = loss_coefficients(n, p.moments[0], p.moments[1], p.moments[2], p.moments[3], p.moments[4],
+                                              (double)p.w_mse, (double)p.w_ncc);
+        p.loss_log[p.epoch] = (float)(lc.loss + (double)w_lncc * lncc_stats[1] + (double)p.lambda * p.moments[5]);
+    }
+    const float sw[3] = {2.f * p.lambda * smooth_weight<NDIM>(p, 0), 2.f * p.lambda * smooth_weight<NDIM>(p, 1),
+                         NDIM == 3 ? 2.f * p.lambda * smooth_weight<NDIM>(p, 2) : 0.f};
+    float bc1 = 1.f, bc2s = 1.f;
+    if (p.optimiser == TRB_OPT_ADAM) {
+        bc1 = 1.f - powf(p.beta1, (float)p.step);
+        bc2s = sqrtf(1.f - powf(p.beta2, (float)p.step));
+    }
+    for_each_slab_voxel(Ds, H, W, [&](size_t idx, int x, int y, int zl) {
+        const int z = p.z_off + zl;
+        float f[3] = {0.f, 0.f, 0.f};
+#pragma unroll
+        for (int c = 0; c < NDIM; ++c) f[c] = ld_stream_f(p.flow_in + (size_t)c * slab + idx);
+        float px, py, pz = 0.f;
+        if (NDIM == 3) { pz = flow_pos(az, z, f[0]); py = flow_pos(ay, y, f[1]); px = flow_pos(ax, x, f[2]); }
+        else { py = flow_pos(ay, y, f[0]); px = flow_pos(ax, x, f[1]); }
+        const Sample<NDIM> sp = sample_zero_pad<NDIM, true>(p.moving, D, H, W, px, py, pz);
+        const float g[3] = {sp.g[0], sp.g[1], NDIM == 3 ? sp.g[NDIM - 1] : 0.f};
+        const float r = ld_stream_f(resid + idx);
+#pragma unroll
+        for (int c = 0; c < NDIM; ++c) {
+            float gr = r * g[NDIM - 1 - c];          // channel c <-> sampling coordinate NDIM-1-c
+            if (p.lambda != 0.f) {
+                float st = 0.f;
+                if (x + 1 < W) st -= sw[0] * (flow_at<NDIM>(p, c, zl, y, x + 1) - f[c]);
+                if (x > 0) st += sw[0] * (f[c] - flow_at<NDIM>(p, c, zl, y, x - 1));
+                if (y + 1 < H) st -= sw[1] * (flow_at<NDIM>(p, c, zl, y + 1, x) - f[c]);
+                if (y > 0) st += sw[1] * (f[c] - flow_at<NDIM>(p, c, zl, y - 1, x));
+                if (NDIM == 3) {
+                    if (z + 1 < D) st -= sw[2] * (flow_at<NDIM>(p, c, zl + 1, y, x) - f[c]);
+                    if (z > 0) st += sw[2] * (f[c] - flow_at<NDIM>(p, c, zl - 1, y, x));
+                }
+                gr += st;
+            }
+            const size_t o = (size_t)c * slab + idx;
+            float nv;
+            if (p.optimiser == TRB_OPT_SGD) {
+                nv = f[c] - p.lr * gr;
+            } else {
+                float m = p.adam_m[o], v = p.adam_v[o];
+                m = p.beta1 * m + (1.f - p.beta1) * gr;
+                v = p.beta2 * v + (1.f - p.beta2) * gr * gr;
+                p.adam_m[o] = m; p.adam_v[o] = v;
+                nv = f[c] - (p.lr / bc1) * (m / (sqrtf(v) / bc2s + p.eps));
+            }
+            p.flow_out[o] = nv;
+        }
+    });
+}
+
 // ---- fused single-pass epoch (3-D) -------------------------------------------------------------------------
 // One kernel per epoch instead of two.  A CTA owns a 32x8 (x,y) tile and marches along z over a chunk of
 // slices: the z-1 / z / z+1 flow values of a voxel are the thread's own registers (sliding window), the x+-1 /
@@ -689,8 +755,44 @@ extern "C" int trb_flow_direct_update(int ndim, const float *moving_dev, const f
     return check_cuda(cudaGetLastError(), "flow_direct_update");
 }
 
+extern "C" int trb_flow_direct_update_lncc(int ndim, const float *moving_dev, const float *flow_in_dev, float *flow_out_dev,
+                                           const float *resid_dev, int D, int H, int W, const double *moments6_dev,
+                                           const double *lncc_stats_dev, float w_mse, float w_ncc, float w_lncc,
+                                           float smooth_lambda, float lr, int optimiser, float beta1, float beta2,
+                                           float adam_eps, int step_index, float *adam_m_dev, float *adam_v_dev,
+                                           float *loss_log_dev, int epoch, void *stream)
+{
+    DirectParams p{};
+    if (ndim != 2 && ndim != 3) { set_error("ndim must be 2 or 3"); return TRB_ERR_ARG; }
+    if (ndim == 2) D = 1;
+    if (H < 2 || W < 2 || (ndim == 3 && D < 2)) { set_error("flow needs every axis >= 2"); return TRB_ERR_ARG; }
+    if (int rc = check_fast_floor_axes(ndim, D, H, W)) return rc;
+    if ((unsigned long long)D * H * W >= (1ull << 31)) { set_error("flow kernels index volumes with 32 bits: D*H*W must stay below 2^31"); return TRB_ERR_ARG; }
+    if (!moving_dev || !flow_in_dev || !flow_out_dev || !resid_dev || !moments6_dev || !lncc_stats_dev) { set_error("null pointer"); return TRB_ERR_ARG; }
+    const size_t vol = (size_t)D * H * W, fb = (size_t)ndim * vol * sizeof(float);
+    const char *fi = (const char *)flow_in_dev, *fo = (const char *)flow_out_dev, *rr = (const char *)resid_dev;
+    if ((fo < fi + fb && fi < fo + fb) || (fo < rr + vol * sizeof(float) && rr < fo + fb)) {
+        set_error("update is out of place: flow_out must not overlap flow_in or the residual");
+        return TRB_ERR_ARG;
+    }
+    if (optimiser != TRB_OPT_SGD && optimiser != TRB_OPT_ADAM) { set_error("bad optimiser"); return TRB_ERR_ARG; }
+    if (optimiser == TRB_OPT_ADAM && (!adam_m_dev || !adam_v_dev || step_index < 1)) { set_error("Adam needs m, v and step_index >= 1"); return TRB_ERR_ARG; }
+    p.moving = moving_dev; p.flow_in = flow_in_dev; p.flow_out = flow_out_dev;
+    p.D = D; p.H = H; p.W = W; p.z_off = 0; p.Ds = D;
+    p.moments = const_cast<double *>(moments6_dev);
+    p.w_mse = w_mse; p.w_ncc = w_ncc; p.lambda = smooth_lambda; p.lr = lr;
+    p.optimiser = optimiser; p.beta1 = beta1; p.beta2 = beta2; p.eps = adam_eps; p.step = step_index;
+    p.adam_m = adam_m_dev; p.adam_v = adam_v_dev; p.loss_log = loss_log_dev; p.epoch = epoch;
+    unsigned g;
+    if (int rc = direct_grid(vol, g)) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (ndim == 3) flow_direct_update_lncc_kernel<3><<<g, 256, 0, s>>>(p, resid_dev, lncc_stats_dev, w_lncc);
+    else flow_direct_update_lncc_kernel<2><<<g, 256, 0, s>>>(p, resid_dev, lncc_stats_dev, w_lncc);
+    return check_cuda(cudaGetLastError(), "flow_direct_update_lncc");
+}
+
 namespace trb {
-static int g_step_no_tma = 0;        // trb_flow_direct_set_path: 1 = register-staged kernel for the smoothness variants too (A/B)
+static int g_step_no_tma = 0;       // trb_flow_direct_set_path: 1 = register-staged kernel for the smoothness variants too (A/B)
 template <bool NEXT, bool ADAM>
 static void launch_step(const DirectParams &p, bool smooth, unsigned grid, int tiles_x, int tiles_y, int zc, cudaStream_t s)
 {

@@ -497,6 +497,77 @@ def flow_loss_grad(moving: torch.Tensor, target: torch.Tensor, flow: torch.Tenso
 
 
 # --------------------------------------------------------------------------- #
+# EXTENSION: local normalised cross-correlation (csrc/lncc.cu; no reference counterpart)
+# --------------------------------------------------------------------------- #
+LNCC_MAX_WIN = 15
+_LNCC_WS = {}
+
+
+def check_lncc_window(win: int) -> int:
+    if isinstance(win, bool) or int(win) != win or win < 3 or win > LNCC_MAX_WIN or win % 2 == 0:
+        raise ValueError("the LNCC window must be an odd integer in [3, %d] (got %r)" % (LNCC_MAX_WIN, win))
+    return int(win)
+
+
+def check_lncc_pair(target: torch.Tensor, warped: torch.Tensor):
+    """CUDA fp32 [N,1,(D,)H,W] pairs of one shape -> (ndim, N, D, H, W); raises otherwise (there is no CPU path)."""
+    for t, name in ((target, "target"), (warped, "warped")):
+        if isinstance(t, torch.Tensor) and t.dtype != torch.float32:
+            raise TypeError("%s must be float32 (got %s)" % (name, t.dtype))
+    require_cuda(target, "target")
+    require_cuda(warped, "warped")
+    ndim, D, H, W = _vol_dims(warped)
+    if warped.shape[1] != 1 or target.shape != warped.shape:
+        raise ValueError("LNCC expects target and warped of one [N,1,...] shape (got %s and %s)"
+                         % (tuple(target.shape), tuple(warped.shape)))
+    return ndim, int(warped.shape[0]), D, H, W
+
+
+def _lncc_ws(dev):
+    ws = _LNCC_WS.get(str(dev))
+    if ws is None:
+        ws = torch.zeros(int(_lib.load().trb_lncc_workspace_bytes()), dtype=torch.uint8, device=dev)
+        _LNCC_WS[str(dev)] = ws
+    return ws
+
+
+def lncc_forward(target: torch.Tensor, warped: torch.Tensor, win: int = 9, eps: float = 1e-5):
+    """-> (stats [2] fp64 device tensor (sum of cc, loss), coef [3, N*D*H*W] = alpha, beta, gamma) for
+    loss = 1 - mean(cc) of the windowed NCC (include/trb.h: trb_lncc_forward)."""
+    win = check_lncc_window(win)
+    ndim, n, D, H, W = check_lncc_pair(target, warped)
+    dev = warped.device
+    t, w = target.detach().contiguous(), warped.detach().contiguous()
+    coef = torch.empty(3, t.numel(), dtype=torch.float32, device=dev)
+    stats = torch.empty(2, dtype=torch.float64, device=dev)
+    ws = _lncc_ws(dev)
+    with torch.cuda.device(dev):
+        check(_lib.load().trb_lncc_forward(ndim, t.data_ptr(), w.data_ptr(), n, D, H, W, win, float(eps), coef.data_ptr(),
+                                           stats.data_ptr(), ws.data_ptr(), ws.numel(), _stream(dev)), "lncc_forward")
+    return stats, coef
+
+
+def lncc_backward(target: torch.Tensor, warped: torch.Tensor, coef: torch.Tensor, win: int = 9, scale: float = 1.0) -> torch.Tensor:
+    """scale * d loss / d warped for the coef of lncc_forward on the same pair and window."""
+    win = check_lncc_window(win)
+    ndim, n, D, H, W = check_lncc_pair(target, warped)
+    dev = warped.device
+    t, w = target.detach().contiguous(), warped.detach().contiguous()
+    grad = torch.empty_like(w)
+    with torch.cuda.device(dev):
+        check(_lib.load().trb_lncc_backward(ndim, t.data_ptr(), w.data_ptr(), coef.data_ptr(), n, D, H, W, win, float(scale),
+                                            None, 0.0, 0.0, grad.data_ptr(), _stream(dev)), "lncc_backward")
+    return grad
+
+
+def lncc_loss_grad(warped: torch.Tensor, target: torch.Tensor, win: int = 9, eps: float = 1e-5):
+    """-> (loss, d loss / d warped): loss = 1 - mean(cc) of the windowed NCC of (target, warped) as a 0-dim fp32 device
+    tensor, and its gradient (two kernels, no host synchronisation)."""
+    stats, coef = lncc_forward(target, warped, win, eps)
+    return stats[1].float(), lncc_backward(target, warped, coef, win)
+
+
+# --------------------------------------------------------------------------- #
 # EXTENSION: direct per-voxel flow optimisation (no reference counterpart)
 # --------------------------------------------------------------------------- #
 class NmiTerm:
@@ -893,8 +964,13 @@ class DirectFlowProblem:
         self._pending = False
         self._sums_epoch = self.epoch if w_ncc != 0 else -1      # moments[0..4] describe the current flow
 
-    def run(self, n_epochs, lr, w_mse, w_ncc, smooth=0.0, betas=(0.9, 0.999), eps=1e-8):
-        """Single-GPU epochs (whole volume in this problem): no host synchronisation."""
+    def run(self, n_epochs, lr, w_mse, w_ncc, smooth=0.0, betas=(0.9, 0.999), eps=1e-8, *, w_lncc=0.0, lncc_win=9,
+            lncc_eps=1e-5):
+        """Single-GPU epochs (whole volume in this problem): no host synchronisation.  w_lncc != 0 adds the local NCC
+        term (window lncc_win) and runs `run_lncc`'s epochs."""
+        if w_lncc != 0:
+            self.run_lncc(n_epochs, lr, w_mse, w_ncc, w_lncc, lncc_win, lncc_eps, smooth, betas, eps)
+            return
         if self.fused and n_epochs > 0:
             self.prime(w_ncc)
             for _ in range(n_epochs):
@@ -904,6 +980,50 @@ class DirectFlowProblem:
         for _ in range(n_epochs):
             self.stats(smooth)
             self.update(lr, w_mse, w_ncc, smooth, betas=betas, eps=eps)
+
+    def run_lncc(self, n_epochs, lr, w_mse, w_ncc, w_lncc, win=9, lncc_eps=1e-5, smooth=0.0, betas=(0.9, 0.999), eps=1e-8):
+        """Epochs of loss = w_lncc * (1 - mean cc) + w_mse*MSE + w_ncc*100*(1-NCC) + smooth * R(flow), whole volume on one
+        GPU, no host synchronisation.  Per epoch: the stats pass (MSE / NCC moments and the smoothness sum; skipped when
+        all three weights are 0), the flow warp J, trb_lncc_forward, trb_lncc_backward (dL/dJ, with the pointwise MSE /
+        NCC terms) and trb_flow_direct_update_lncc.  loss_log[e] is the loss of flow_e, before its step."""
+        win = check_lncc_window(win)
+        if self.ndim == 3 and (self.z_off != 0 or self.Ds != self.D):
+            raise ValueError("the LNCC epoch runs on the whole volume (no z-slab)")
+        if self.epoch + n_epochs > self.max_epochs:
+            raise ValueError("max_epochs exceeded")
+        if getattr(self, "_lncc", None) is None:
+            # J, alpha / beta / gamma and dL/dJ: 5 volumes (335 MB at 256^3), kept for the problem's lifetime
+            self._lncc = (torch.empty_like(self.target), torch.empty(3, self.target.numel(), dtype=torch.float32, device=self.device),
+                          torch.empty_like(self.target), torch.zeros(2, dtype=torch.float64, device=self.device),
+                          torch.zeros(int(self.lib.trb_lncc_workspace_bytes()), dtype=torch.uint8, device=self.device))
+        warped, coef, resid, lstats, lws = self._lncc
+        need_stats = w_mse != 0 or w_ncc != 0 or smooth != 0
+        if not need_stats:
+            self.moments.zero_()
+        lib, s = self.lib, _stream(self.device)
+        with torch.cuda.device(self.device):
+            for _ in range(n_epochs):
+                if need_stats:
+                    self.stats(smooth)
+                check(lib.trb_warp_flow(self.ndim, self.moving.data_ptr(), self.flow.data_ptr(), warped.data_ptr(), 1,
+                                        self.D, self.H, self.W, s), "warp_flow")
+                check(lib.trb_lncc_forward(self.ndim, self.target.data_ptr(), warped.data_ptr(), 1, self.D, self.H, self.W,
+                                           win, float(lncc_eps), coef.data_ptr(), lstats.data_ptr(), lws.data_ptr(),
+                                           lws.numel(), s), "lncc_forward")
+                check(lib.trb_lncc_backward(self.ndim, self.target.data_ptr(), warped.data_ptr(), coef.data_ptr(), 1,
+                                            self.D, self.H, self.W, win, float(w_lncc),
+                                            self.moments.data_ptr() if (w_mse != 0 or w_ncc != 0) else None,
+                                            float(w_mse), float(w_ncc), resid.data_ptr(), s), "lncc_backward")
+                check(lib.trb_flow_direct_update_lncc(
+                    self.ndim, self.moving.data_ptr(), self.flow.data_ptr(), self._other.data_ptr(), resid.data_ptr(),
+                    self.D, self.H, self.W, self.moments.data_ptr(), lstats.data_ptr(), float(w_mse), float(w_ncc),
+                    float(w_lncc), float(smooth), float(lr), OPT[self.optimiser], float(betas[0]), float(betas[1]),
+                    float(eps), self.epoch + 1, _ptr(self.adam_m), _ptr(self.adam_v), self.loss_log.data_ptr(), self.epoch,
+                    s), "flow_direct_update_lncc")
+                self.flow, self._other = self._other, self.flow
+                self.epoch += 1
+        self._pending = False
+        self._sums_epoch = -1          # moments describe the flow before the last step
 
     def run_two_pass(self, n_epochs, lr, w_mse, w_ncc, smooth=0.0, betas=(0.9, 0.999), eps=1e-8):
         """The stats + update form of `run` (2-D, very large slabs, and the cross-check of the fused kernel)."""

@@ -19,7 +19,7 @@ from . import functional as TF
 
 EPSILON = 1E-10
 
-__all__ = ["EPSILON", "NCCLoss", "SSDLoss", "NMILoss", "norm", "padNd", "Theta", "Regressor", "SpatialTransformer",
+__all__ = ["EPSILON", "NCCLoss", "LNCCLoss", "SSDLoss", "NMILoss", "norm", "padNd", "Theta", "Regressor", "SpatialTransformer",
            "attention_grid", "Attention_UNet", "Edge3D", "get_sobel_kernel3D"]
 
 
@@ -42,6 +42,44 @@ class NCCLoss(nn.Module):
         b = yp - torch.mean(yp)
         self.NCC = torch.sum(a * b) / ((torch.sum(a ** 2) * torch.sum(b ** 2) + EPSILON) ** 0.5)
         return (1 - self.NCC) * self.alpha
+
+
+class LNCCLoss(nn.Module):
+    """EXTENSION (no counterpart in the reference): local (windowed) normalised cross-correlation, VoxelMorph's NCC with
+    the sign turned so the loss is >= 0: loss = 1 - mean over all voxels of cc, cc = A^2 / (B C + eps) over a win^nd box
+    with zero padding (include/trb.h: trb_lncc_forward).  forward(y, yp) = crit(target, warped), the order of the
+    reference's criteria; the gradient flows to yp only.  CUDA fp32 [N,1,(D,)H,W] only, on the kernels of csrc/lncc.cu.
+    Recognised by type in direct flow mode, where it runs inside the epoch."""
+
+    def __init__(self, win=9, eps=1e-5):
+        super().__init__()
+        self.win = TF.check_lncc_window(win)
+        if not (float(eps) > 0 and float(eps) < float('inf')):
+            raise ValueError("eps must be finite and > 0 (got %r)" % (eps,))
+        self.eps = float(eps)
+
+    def forward(self, y, yp):
+        if isinstance(y, torch.Tensor) and y.requires_grad:
+            raise ValueError("LNCCLoss differentiates w.r.t. the warped image yp only: y (the target) must not require grad")
+        TF.check_lncc_pair(y, yp)
+        return _LnccFn.apply(yp, y, self.win, self.eps)
+
+
+class _LnccFn(torch.autograd.Function):
+    """autograd node: forward = trb_lncc_forward (keeps alpha, beta, gamma), backward = trb_lncc_backward."""
+
+    @staticmethod
+    def forward(ctx, yp, y, win, eps):
+        stats, coef = TF.lncc_forward(y, yp, win, eps)
+        ctx.win = win
+        if ctx.needs_input_grad[0]:
+            ctx.save_for_backward(y, yp, coef)
+        return stats[1].float()
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        y, yp, coef = ctx.saved_tensors
+        return TF.lncc_backward(y, yp, coef, ctx.win) * grad_out, None, None, None
 
 
 class SSDLoss(nn.Module):

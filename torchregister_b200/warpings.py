@@ -14,7 +14,7 @@ import torch
 import torch.nn as nn
 
 from . import functional as TF
-from .utils import Attention_UNet, NCCLoss, NMILoss
+from .utils import Attention_UNet, LNCCLoss, NCCLoss, NMILoss
 
 __all__ = ["get_affine_warp", "affine_register", "rigid_register", "flow_register", "direct_flow_register",
            "similarity_weights", "compose_theta"]
@@ -247,6 +247,18 @@ def _split_criteria(criterions, weights):
     return w_mse, w_ncc, other
 
 
+def _split_lncc(other):
+    """-> (w_lncc, win, eps, rest): the summed weight of the LNCCLoss terms among `other` (the third result of
+    _split_criteria), their window and eps, and the remaining terms.  Every LNCCLoss term must share one window and eps."""
+    terms = [(wt, crit) for wt, crit in other if isinstance(crit, LNCCLoss)]
+    rest = [(wt, crit) for wt, crit in other if not isinstance(crit, LNCCLoss)]
+    if not terms:
+        return 0.0, 9, 1e-5, rest
+    if len({(crit.win, crit.eps) for _, crit in terms}) > 1:
+        raise NotImplementedError("direct flow takes LNCCLoss terms with one window and eps only")
+    return sum(float(wt) for wt, _ in terms), terms[0][1].win, terms[0][1].eps, rest
+
+
 class _FlowSimilarityFn(torch.autograd.Function):
     """loss = w_mse*MSE(target, warp(moving, flow)) + w_ncc*100*(1-NCC(...)), fused with its
     gradient w.r.t. flow (one statistics pass + one gradient pass over the volume)."""
@@ -374,7 +386,8 @@ class direct_flow_register:
     parameter, optimised with SGD or Adam on  sum_i w_i*crit_i(target, warp(moving, flow)) + smooth * R(flow),
     R = mean over axes of the mean squared forward difference.  Same duck type as `flow_register`
     (`optimize`, `deform`, `flow`, `losses`) so `Register(mode='flow', flow_param='direct')` can swap it in.
-    Only nn.MSELoss / NCCLoss terms are supported (they are what the fused kernels evaluate)."""
+    Only nn.MSELoss, NCCLoss and LNCCLoss terms are supported (they are what the kernels evaluate).  With an LNCCLoss
+    term every epoch runs the local-NCC form (functional.DirectFlowProblem.run_lncc); without one, the fused epoch."""
 
     def __init__(self, img_size, criterions=None, weights=[0.5, 0.5], lr=1E-3, max_epochs=2000, stop_crit=1E-4,
                  smooth=0.0, optimiser='sgd', betas=(0.9, 0.999), eps=1e-8):
@@ -384,8 +397,9 @@ class direct_flow_register:
                 raise NotImplementedError("direct flow supports the MSE and NCC terms only (weight[2] must be 0)")
             weights = list(weights)[:2]
         self.w_mse, self.w_ncc, other = _split_criteria(criterions, weights)
+        self.w_lncc, self.lncc_win, self.lncc_eps, other = _split_lncc(other)
         if other:
-            raise NotImplementedError("direct flow supports nn.MSELoss and NCCLoss criteria only")
+            raise NotImplementedError("direct flow supports nn.MSELoss, NCCLoss and LNCCLoss criteria only")
         self.img_size = tuple(img_size)
         self.lr, self.max_epochs, self.stop_crit = lr, max_epochs, stop_crit
         self.smooth, self.optimiser, self.betas, self.eps = smooth, optimiser.lower(), betas, eps
@@ -405,7 +419,8 @@ class direct_flow_register:
         chunk = check_every
         while done < self.max_epochs:
             n = min(chunk, self.max_epochs - done)
-            prob.run(n, self.lr, self.w_mse, self.w_ncc, self.smooth, self.betas, self.eps)
+            prob.run(n, self.lr, self.w_mse, self.w_ncc, self.smooth, self.betas, self.eps, w_lncc=self.w_lncc,
+                     lncc_win=self.lncc_win, lncc_eps=self.lncc_eps)
             done += n
             lo = prob.losses[done - n:done]
             hit = (lo <= self.stop_crit).nonzero()
